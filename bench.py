@@ -20,6 +20,8 @@ between the GPU and the CPU arms; `ms_per_step` is the ordering's wall time.
   cpu_baseline / --impl reference: the CPU restatement of the reference (oracle/, "port": the JAR
             cannot run here - no JVM) on bounded samples, all host threads and 1 thread, with the
             c*n^3 fit that extrapolates the CPU wall time to the workload's n.
+  --dump-outputs DIR  the ordering the timed path returned in its last step, as DIR/ordering.npy (float64), so
+            that two builds can be compared output for output: the inputs are seeded, the same on every run.
 
 N>1: one process per GPU, ONE job (fixed total work -> "strong" scaling at every N): the selection
 scan (the Theta(n^3) part) is sharded across the ranks, the per-rank (Q,i,j) partial min-locs are
@@ -63,6 +65,15 @@ def cpu_reference_run(n, seed, threads, want_order=False):
     o, _, info = oracle.order(D, mode="canonical", want_trace=False, threads=threads)
     dt = time.perf_counter() - t0
     return (dt, info["alg_bytes"], o) if want_order else (dt, info["alg_bytes"])
+
+
+def dump_outputs(directory, **arrays):
+    """--dump-outputs: each array as float64 DIR/<name>.npy (an int32 ordering is exact in float64; n+1 entries stay far
+    below 64 MB at any n whose matrix fits a GPU)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def cubic_fit(ns, ts):
@@ -159,9 +170,11 @@ def run_reference(args, rank, world, emit=None):
         cpu_reference_run(n, 100 + i, threads)
     tot_t, tot_b = 0.0, 0.0
     for i in range(args.steps):
-        dt, b = cpu_reference_run(n, 1 + i, threads)
+        dt, b, o = cpu_reference_run(n, 1 + i, threads, want_order=True)
         tot_t += dt
         tot_b += b
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ordering=o)
     val = tot_b / tot_t / 1e9
     ms = 1e3 * tot_t / args.steps
     # c*n^3 fits (BASELINE.md section 4.3): all threads on --fit-n, 1 thread on --fit-n1
@@ -214,7 +227,10 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--csw-n", type=int, default=400, help="taxa of the split-weight config entry")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's ordering to DIR/ordering.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -335,6 +351,8 @@ def main():
     clocks = sampler.stop() if sampler else None
     if ordering0 is not None:
         assert (o == ordering0).all(), "ordering changed between identical steps"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ordering=o)
     picks = (st["picks_certified"], st["picks_exact"])
     # max over ranks of the elapsed time; launches summed over ranks
     if world > 1:

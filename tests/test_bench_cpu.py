@@ -25,6 +25,27 @@ def test_reference_arm_line():
     assert ex["threads_1"]["seconds_at_workload_n"] >= ex["threads_all"]["seconds_at_workload_n"] * 0.2
 
 
+def test_reference_arm_dumps_last_step_ordering(tmp_path):
+    """--dump-outputs writes what the last timed step computed: with --steps 2 that is the ordering of seed 2's matrix."""
+    import numpy as np
+    import oracle
+    from fastneighbornet_b200 import synth
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "0",
+                        "--ref-n", "120", "--fit-n", "120", "--fit-n1", "100", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = np.load(tmp_path / "ordering.npy")
+    assert got.dtype == np.float64
+    o_ref, _, _ = oracle.order(synth.additive_noise_matrix(120, 2, 0.05), want_trace=False)
+    assert (got == o_ref).all()
+
+
+def test_zero_steps_is_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=60)
+    assert r.returncode == 2 and "--steps" in r.stderr
+
+
 def test_cubic_fit():
     sys.path.insert(0, ROOT)
     import bench
