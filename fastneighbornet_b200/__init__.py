@@ -19,6 +19,7 @@ from .api import (  # noqa: F401
     rowsums,
     seq_sum,
     split_weights,
+    split_weights_budget,
     csw_matvec,
     weighted_splits,
     network_splits,

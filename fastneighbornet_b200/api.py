@@ -61,7 +61,7 @@ ABI_SYMBOLS = [
     "fnn_ctx_trace", "fnn_ctx_stats", "fnn_ctx_matrix_ptr", "fnn_order", "fnn_rowsums", "fnn_seq_sum",
     "fnn_split_weights", "fnn_csw_matvec", "fnn_ctx_ipc_handle", "fnn_ctx_connect", "fnn_weighted_splits", "fnn_network",
     "fnn_phylip_taxa", "fnn_read_phylip", "fnn_write_nexus", "fnn_java_double_to_string", "fnn_release_cache",
-    "fnn_ctx_load_host_rows", "fnn_ctx_commit_load",
+    "fnn_ctx_load_host_rows", "fnn_ctx_commit_load", "fnn_split_weights_budget",
 ]
 
 
@@ -105,6 +105,9 @@ def lib():
         L.fnn_rowsums.argtypes = [ctypes.POINTER(fnn_opts), c_dp, ctypes.c_int64, c_dp]
         L.fnn_split_weights.argtypes = [ctypes.POINTER(fnn_opts), ctypes.POINTER(ctypes.c_int32), c_dp, ctypes.c_int64, c_dp,
                                         ctypes.POINTER(ctypes.c_int64)]
+        L.fnn_split_weights_budget.argtypes = [ctypes.POINTER(fnn_opts), ctypes.POINTER(ctypes.c_int32), c_dp, ctypes.c_int64,
+                                               ctypes.c_int64, ctypes.c_int64, c_dp, ctypes.POINTER(ctypes.c_uint8),
+                                               ctypes.POINTER(ctypes.c_int64)]
         L.fnn_weighted_splits.argtypes = [ctypes.POINTER(fnn_opts), ctypes.POINTER(ctypes.c_int32), c_dp, ctypes.c_int64, ctypes.c_double,
                                           ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32), c_dp, ctypes.c_int64,
                                           ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]
@@ -345,6 +348,27 @@ def split_weights(ordering, d_upper, constrained=True, variant="default", **opts
     _check(lib().fnn_split_weights(ctypes.byref(o), ordering.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), _dp(d_upper), n,
                                    _dp(x), st.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
     return x, {"cg_iters": int(st[0]), "cg_calls": int(st[1]), "outer": int(st[2]), "inner": int(st[3]), "kernel_launches": int(st[4])}
+
+
+def split_weights_budget(ordering, d_upper, max_cg_iters=0, max_cg_calls=0, variant="default", **opts):
+    """fnn_split_weights_budget: split_weights with every CG call capped at max_cg_iters iterations and the solver stopped
+    right after its max_cg_calls-th CG call (0 = no limit; both 0 = split_weights).  For parity tests at production sizes.
+    Returns (x[npairs], active[npairs] bool, stats dict as split_weights)."""
+    opts = dict(opts, csw_variant=CSW_VARIANTS[variant])
+    ordering = np.ascontiguousarray(ordering, dtype=np.int32)
+    n = ordering.shape[0] - 1
+    d_upper = np.ascontiguousarray(d_upper, dtype=np.float64)
+    assert d_upper.shape[0] == n * (n - 1) // 2
+    o = default_opts(**opts)
+    x = np.zeros_like(d_upper)
+    active = np.zeros(d_upper.shape[0], dtype=np.uint8)
+    st = np.zeros(5, dtype=np.int64)
+    _check(lib().fnn_split_weights_budget(ctypes.byref(o), ordering.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), _dp(d_upper), n,
+                                          int(max_cg_iters), int(max_cg_calls), _dp(x),
+                                          active.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)),
+                                          st.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
+    return x, active.astype(bool), {"cg_iters": int(st[0]), "cg_calls": int(st[1]), "outer": int(st[2]), "inner": int(st[3]),
+                                    "kernel_launches": int(st[4])}
 
 
 def network_splits(ordering, d_upper, cutoff=1e-6, constrained=True, **opts):

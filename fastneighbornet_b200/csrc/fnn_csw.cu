@@ -1158,7 +1158,7 @@ k_cg(int n, int np, double* r, double* w, double* p, double* y, const double* b,
     xsum::Smem* sm = reinterpret_cast<xsum::Smem*>(smem_raw);
     __shared__ double res[1];
     const int tid = threadIdx.x;
-    const long long kmax = (long long)n * (n - 1) / 2;
+    const long long kmax = sc->kmax;   // npairs, or the test budget of fnn_split_weights_budget
     ab(n, x, y);
     atx(n, y, r);
     for (int k = tid; k < np; k += THREADS) r[k] = active[k] ? 0.0 : b[k] - r[k];
@@ -1204,6 +1204,11 @@ struct Csw {
     Scalars* h_sc = nullptr;
     cudaGraphExec_t cg_graph = nullptr;
     int64_t cg_calls = 0, outer = 0, inner = 0, launches = 0, launches_per_graph = 0;
+    // CG iteration cap of every circularConjugateGrads call (kmax of :795, uploaded to Scalars::kmax): npairs, or
+    // min(npairs, max_cg_iters) under the budget of fnn_split_weights_budget; max_cg_calls > 0 stops the active-set method
+    // right after that many CG calls.  0 = no budget (production).
+    long long kmax = 0, max_cg_iters = 0, max_cg_calls = 0;
+    bool budget_spent() const { return max_cg_calls > 0 && cg_calls >= max_cg_calls; }
     std::chrono::steady_clock::time_point t_start = std::chrono::steady_clock::now();
     double t_progress = 0.0;
     int persistent = 0;        // 1: k_cg_persistent (one cooperative launch per CG solve) instead of the graph path
@@ -1428,17 +1433,24 @@ static int active_conjugate(Csw& c) {
         k_square_partials<<<(unsigned)c.nblk, 256, 0, c.st>>>(c.AtWd, c.np, c.part1);
         c.finish_tree(EP_E0, 0);
     }
-    FNN_CUDA(cudaMemcpyAsync(&c.sc->kmax, &c.np, sizeof(long long), cudaMemcpyHostToDevice, c.st));
+    c.kmax = c.max_cg_iters > 0 ? std::min<long long>(c.np, c.max_cg_iters) : (long long)c.np;
+    FNN_CUDA(cudaMemcpyAsync(&c.sc->kmax, &c.kmax, sizeof(long long), cudaMemcpyHostToDevice, c.st));
     bool first_pass = true;
     while (true) {
         ++c.outer;
         while (true) {
             ++c.inner;
-            if (!first_pass) { if (c.conjugate_grads()) return FNN_E_CUDA; }
+            if (!first_pass) {
+                if (c.conjugate_grads()) return FNN_E_CUDA;
+                if (c.budget_spent()) return FNN_OK;
+            }
             first_pass = false;
             bool contracted = false;
             if (contract_worst(c, &contracted)) return FNN_E_CUDA;
-            if (contracted) { if (c.conjugate_grads()) return FNN_E_CUDA; }
+            if (contracted) {
+                if (c.conjugate_grads()) return FNN_E_CUDA;
+                if (c.budget_spent()) return FNN_OK;
+            }
             if (minloc_reduce(c, RatioIn{c.x, c.old_x}, &ml)) return FNN_E_CUDA;
             if (ml.i < 0) break;
             k_oldx_step<<<c.grid1d(c.np, 256), 256, 0, c.st>>>(c.old_x, c.x, c.active, c.np, ml.v);
@@ -1555,6 +1567,33 @@ extern "C" int fnn_split_weights(const fnn_opts* o, const int32_t* ordering, con
     if (!rc && cudaMemcpyAsync(x_out, c.x, sizeof(double) * c.np, cudaMemcpyDeviceToHost, c.st) != cudaSuccess) {
         fnn::set_error("fnn_split_weights: %s", cudaGetErrorString(cudaGetLastError()));
         rc = FNN_E_CUDA;
+    }
+    if (!rc) rc = fetch_stats(c, stats_out);
+    c.release();
+    return rc;
+}
+
+extern "C" int fnn_split_weights_budget(const fnn_opts* o, const int32_t* ordering, const double* d_upper, int64_t n,
+                                        int64_t max_cg_iters, int64_t max_cg_calls, double* x_out, uint8_t* active_out,
+                                        int64_t* stats_out) {
+    int rc = check_b2_args(o, ordering, d_upper, n);
+    if (rc) return rc;
+    if (!x_out || !active_out || max_cg_iters < 0 || max_cg_calls < 0) {
+        fnn::set_error("fnn_split_weights_budget: null output or negative budget");
+        return FNN_E_ARG;
+    }
+    Csw c;
+    c.max_cg_iters = max_cg_iters;
+    c.max_cg_calls = max_cg_calls;
+    rc = solve_split_weights(c, o, ordering, d_upper, n);
+    if (!rc) {
+        // the mask is set up when the active-set loop is entered (outer > 0); before that every split is free
+        if (c.outer == 0) memset(active_out, 0, (size_t)c.np);
+        if (cudaMemcpyAsync(x_out, c.x, sizeof(double) * c.np, cudaMemcpyDeviceToHost, c.st) != cudaSuccess ||
+            (c.outer > 0 && cudaMemcpyAsync(active_out, c.active, (size_t)c.np, cudaMemcpyDeviceToHost, c.st) != cudaSuccess)) {
+            fnn::set_error("fnn_split_weights_budget: %s", cudaGetErrorString(cudaGetLastError()));
+            rc = FNN_E_CUDA;
+        }
     }
     if (!rc) rc = fetch_stats(c, stats_out);
     c.release();

@@ -185,6 +185,19 @@ int fnn_network(const fnn_opts* o, const double* D_rowmajor, int64_t n, double c
  * 2: unconstrained closed form (runUnconstrainedLS, :247-271) */
 int fnn_csw_matvec(const fnn_opts* o, int32_t which, const double* v, int64_t n, double* out);
 
+/* fnn_split_weights under an iteration budget, for parity tests at sizes whose full solve takes minutes to hours (the same
+ * solver, variant selection by opts.reserved[4] included; the production entry points never set a budget):
+ *   max_cg_iters = K > 0: every circularConjugateGrads call (CircularSplitWeights.java:769-831) stops after at most K
+ *                         iterations (kmax = min(npairs, K) instead of npairs);
+ *   max_cg_calls = C > 0: the active-set method returns right after its C-th CG call, wherever that call sits in the
+ *                         loop of runActiveConjugate (:359-557).
+ * 0 = no budget; with both 0 the result is that of fnn_split_weights.  The CPU oracles (oracle/csw_l1.cpp L1,
+ * oracle/nnet_oracle.cpp L0) take the same two parameters with the same meaning, so a truncated solve can be compared bit
+ * for bit.  x_out[npairs]: the weights when the solver returned; active_out[npairs]: 1 = split held at zero by the active
+ * set; stats_out (optional, 5 entries) as in fnn_split_weights. */
+int fnn_split_weights_budget(const fnn_opts* o, const int32_t* ordering, const double* d_upper, int64_t n, int64_t max_cg_iters,
+                             int64_t max_cg_calls, double* x_out, uint8_t* active_out, int64_t* stats_out);
+
 /* left-to-right fp64 sums of nrows (<=4) rows of length len, bit-identical to `for (i) s += x[i]`
  * (the accumulation order of ComputeRx / updateClusterDistances, NetMakerOriginal.java:549-561, :530-535),
  * computed by the parallel exact-summation kernel (csrc/fnn_exact_sum.cuh) - exposed for parity tests */

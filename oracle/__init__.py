@@ -41,12 +41,13 @@ def lib():
         L.oracle_unconstrained_ls.argtypes = [ctypes.c_int64, c_dp, c_dp]
         L.oracle_atx.argtypes = [ctypes.c_int64, c_dp, c_dp]
         L.oracle_ab.argtypes = [ctypes.c_int64, c_dp, c_dp]
-        L.oracle_split_weights.argtypes = [ctypes.c_int64, c_dp, c_dp, ctypes.c_int, c_lp]
+        c_bp = ctypes.POINTER(ctypes.c_uint8)
+        L.oracle_split_weights.argtypes = [ctypes.c_int64, c_dp, c_dp, ctypes.c_int, c_lp, ctypes.c_int64, ctypes.c_int64, c_bp]
         L.oracle_l1_ab.argtypes = [ctypes.c_int64, c_dp, c_dp]
         L.oracle_l1_atx.argtypes = [ctypes.c_int64, c_dp, c_dp]
         L.oracle_l1_tree_sum.argtypes = [c_dp, ctypes.c_int64]
         L.oracle_l1_tree_sum.restype = ctypes.c_double
-        L.oracle_l1_split_weights.argtypes = [ctypes.c_int64, c_dp, c_dp, c_lp]
+        L.oracle_l1_split_weights.argtypes = [ctypes.c_int64, c_dp, c_dp, c_lp, ctypes.c_int64, ctypes.c_int64, c_bp]
         L.oracle_set_relaxed_sm.argtypes = [ctypes.c_int]
         L.oracle_java_random.argtypes = [ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, c_ip]
         L.oracle_tile_sequence.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_ip, c_ip, ctypes.c_int64]
@@ -65,6 +66,10 @@ def _ip(a):
 
 def _lp(a):
     return a.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
+
+
+def _bp(a):
+    return a.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
 
 
 def order(D, mode="canonical", seed=12345, mult=5, additive=False, fallback=1024, want_trace=True, threads=1):
@@ -121,12 +126,21 @@ def ab(n, b):
     return _vec(lib().oracle_ab, n, b)
 
 
-def split_weights(n, d_pos, constrained=True):
+def _csw_result(x, st, active, with_active):
+    stats = {"cg_iters": int(st[0]), "cg_calls": int(st[1]), "outer": int(st[2]), "inner": int(st[3])}
+    return (x, active.astype(bool), stats) if with_active else (x, stats)
+
+
+def split_weights(n, d_pos, constrained=True, max_cg_iters=0, max_cg_calls=0, with_active=False):
+    """Parity-ladder level L0: CircularSplitWeights.getWeights in the reference's own operation order (nnet_oracle.cpp).
+    max_cg_iters / max_cg_calls: the budget of fnn_split_weights_budget (0 = none).  Returns (x, stats), or
+    (x, active, stats) with with_active=True."""
     d = np.ascontiguousarray(d_pos, dtype=np.float64)
     x = np.zeros_like(d)
     st = np.zeros(4, dtype=np.int64)
-    lib().oracle_split_weights(n, _dp(d), _dp(x), int(constrained), _lp(st))
-    return x, {"cg_iters": int(st[0]), "cg_calls": int(st[1]), "outer": int(st[2]), "inner": int(st[3])}
+    active = np.zeros(d.shape[0], dtype=np.uint8)
+    lib().oracle_split_weights(n, _dp(d), _dp(x), int(constrained), _lp(st), int(max_cg_iters), int(max_cg_calls), _bp(active))
+    return _csw_result(x, st, active, with_active)
 
 
 def java_random(seed, bound, count):
@@ -157,13 +171,16 @@ def l1_atx(n, d):
     return _vec(lib().oracle_l1_atx, n, d)
 
 
-def l1_split_weights(n, d_pos):
-    """Parity-ladder level L1: the GPU's formulation and reduction trees restated on the CPU (csw_l1.cpp)."""
+def l1_split_weights(n, d_pos, max_cg_iters=0, max_cg_calls=0, with_active=False):
+    """Parity-ladder level L1: the GPU's formulation and reduction trees restated on the CPU (csw_l1.cpp).
+    max_cg_iters / max_cg_calls: the budget of fnn_split_weights_budget (0 = none).  Returns (x, stats), or
+    (x, active, stats) with with_active=True."""
     d = np.ascontiguousarray(d_pos, dtype=np.float64)
     x = np.zeros_like(d)
     st = np.zeros(4, dtype=np.int64)
-    lib().oracle_l1_split_weights(n, _dp(d), _dp(x), _lp(st))
-    return x, {"cg_iters": int(st[0]), "cg_calls": int(st[1]), "outer": int(st[2]), "inner": int(st[3])}
+    active = np.zeros(d.shape[0], dtype=np.uint8)
+    lib().oracle_l1_split_weights(n, _dp(d), _dp(x), _lp(st), int(max_cg_iters), int(max_cg_calls), _bp(active))
+    return _csw_result(x, st, active, with_active)
 
 
 def set_relaxed_sm(on):

@@ -156,7 +156,7 @@ struct Stats { int64_t cg_iters = 0, cg_calls = 0, outer = 0, inner = 0; };
 
 void conjugateGrads(int64_t n, int64_t np, std::vector<double>& r, std::vector<double>& w, std::vector<double>& p,
                     std::vector<double>& y, const std::vector<double>& b, double e0sq, const std::vector<uint8_t>& active,
-                    double* x, Work& wk, Stats& st) {
+                    double* x, int64_t kmax, Work& wk, Stats& st) {
     st.cg_calls++;
     Ab(n, x, y.data(), wk);
     Atx(n, y.data(), r.data(), wk);
@@ -164,7 +164,6 @@ void conjugateGrads(int64_t n, int64_t np, std::vector<double>& r, std::vector<d
     for (int64_t k = 0; k < np; ++k) { const double v = active[k] ? 0.0 : b[k] - r[k]; r[k] = v; sq[k] = v * v; }
     double rho = tree_sum(sq), rho_old = 0.0;
     int64_t k = 0;
-    const int64_t kmax = np;
     while ((rho > e0sq) && (k < kmax)) {
         k = k + 1;
         st.cg_iters++;
@@ -177,6 +176,66 @@ void conjugateGrads(int64_t n, int64_t np, std::vector<double>& r, std::vector<d
         for (int64_t i = 0; i < np; ++i) { x[i] = x[i] + alpha * p[i]; const double rv = r[i] - alpha * w[i]; r[i] = rv; sq[i] = rv * rv; }
         rho_old = rho;
         rho = tree_sum(sq);
+    }
+}
+// runActiveConjugate (:359-557) in the device driver's order (active_conjugate, csrc/fnn_csw.cu).  kmax: iteration cap of
+// every CG call; max_cg_calls > 0: return right after that many CG calls (the budget of fnn_split_weights_budget).
+void activeConjugate(int64_t n, int64_t np, const double* d, double* x, std::vector<uint8_t>& active, int64_t kmax,
+                     int64_t max_cg_calls, Work& wk, Stats& st) {
+    std::vector<double> r(np), w(np), p(np), y(np), old_x(np, 1.0), AtWd(np), sq(np);
+    Atx(n, d, AtWd.data(), wk);
+    for (int64_t k = 0; k < np; ++k) sq[k] = AtWd[k] * AtWd[k];
+    const double e0 = 1e-8 * std::sqrt(tree_sum(sq));
+    const double e0sq = e0 * e0;
+    auto cg = [&]() {
+        conjugateGrads(n, np, r, w, p, y, AtWd, e0sq, active, x, kmax, wk, st);
+        return max_cg_calls > 0 && st.cg_calls >= max_cg_calls;   // budget spent
+    };
+    bool first_pass = true;
+    while (true) {
+        st.outer++;
+        while (true) {
+            st.inner++;
+            if (!first_pass && cg()) return;
+            first_pass = false;
+            {   // worstIndices(x, 0.6) (CircularSplitWeights.java:282-330)
+                std::vector<double> neg;
+                for (int64_t i = 0; i < np; ++i) if (x[i] < 0.0) neg.push_back(x[i]);
+                if (!neg.empty()) {
+                    std::sort(neg.begin(), neg.end());
+                    const int64_t nkept = (int64_t)std::ceil(0.6 * (double)neg.size());
+                    const double cutoff = neg[nkept - 1];
+                    std::vector<int64_t> result(nkept, -1);
+                    int64_t front = 0, back = nkept - 1;
+                    for (int64_t i = 0; i < np; ++i) {
+                        if (x[i] < cutoff) result[front++] = i;
+                        else if (x[i] == cutoff) { if (back >= front) result[back--] = i; }
+                    }
+                    for (int64_t idx : result) if (idx >= 0) { x[idx] = 0.0; active[idx] = 1; }
+                    if (cg()) return;
+                }
+            }
+            int64_t min_i = -1; double min_xi = -1.0;
+            for (int64_t i = 0; i < np; ++i)
+                if (x[i] < 0.0) {
+                    const double xi = old_x[i] / (old_x[i] - x[i]);
+                    if (min_i == -1 || xi < min_xi) { min_i = i; min_xi = xi; }
+                }
+            if (min_i == -1) break;
+            for (int64_t i = 0; i < np; ++i) if (!active[i]) old_x[i] = old_x[i] + min_xi * (x[i] - old_x[i]);
+            active[min_i] = 1;
+            x[min_i] = 0.0;
+        }
+        Ab(n, x, y.data(), wk);
+        Atx(n, y.data(), r.data(), wk);
+        int64_t min_i = -1; double min_grad = 1.0;
+        for (int64_t i = 0; i < np; ++i) {
+            double v = r[i] - AtWd[i];
+            r[i] = v * 2.0;
+            if (active[i]) { if (min_i == -1 || r[i] < min_grad) { min_i = i; min_grad = r[i]; } }
+        }
+        if (min_i == -1 || min_grad > -0.0000001) return;
+        active[min_i] = 0;
     }
 }
 }  // namespace
@@ -194,67 +253,21 @@ void oracle_l1_atx(int64_t n, const double* d, double* p) {
 }
 double oracle_l1_tree_sum(const double* v, int64_t len) { return tree_sum(std::vector<double>(v, v + len)); }
 
-int oracle_l1_split_weights(int64_t n, const double* d, double* x, int64_t* stats) {
+// max_cg_iters / max_cg_calls: the budget of fnn_split_weights_budget (include/fastnn.h), 0 = none.  active_out (optional,
+// npairs bytes): 1 = split held at zero by the active set when the solver returned.
+int oracle_l1_split_weights(int64_t n, const double* d, double* x, int64_t* stats, int64_t max_cg_iters, int64_t max_cg_calls,
+                            uint8_t* active_out) {
     const int64_t np = n * (n - 1) / 2;
     Stats st;
-    Work wk{std::vector<double>(np), std::vector<double>(np), std::vector<double>(n), std::vector<double>(n), std::vector<double>(n)};
+    std::vector<uint8_t> active(np, 0);
     unconstrainedLS(n, d, x);
     bool any_neg = false;
     for (int64_t k = 0; k < np; ++k) if (x[k] < 0.0) { any_neg = true; break; }
     if (any_neg) {
-        std::vector<double> r(np), w(np), p(np), y(np), old_x(np, 1.0), AtWd(np), sq(np);
-        std::vector<uint8_t> active(np, 0);
-        Atx(n, d, AtWd.data(), wk);
-        for (int64_t k = 0; k < np; ++k) sq[k] = AtWd[k] * AtWd[k];
-        const double e0 = 1e-8 * std::sqrt(tree_sum(sq));
-        const double e0sq = e0 * e0;
-        bool first_pass = true;
-        while (true) {
-            st.outer++;
-            while (true) {
-                st.inner++;
-                if (!first_pass) conjugateGrads(n, np, r, w, p, y, AtWd, e0sq, active, x, wk, st);
-                first_pass = false;
-                {   // worstIndices(x, 0.6) (CircularSplitWeights.java:282-330)
-                    std::vector<double> neg;
-                    for (int64_t i = 0; i < np; ++i) if (x[i] < 0.0) neg.push_back(x[i]);
-                    if (!neg.empty()) {
-                        std::sort(neg.begin(), neg.end());
-                        const int64_t nkept = (int64_t)std::ceil(0.6 * (double)neg.size());
-                        const double cutoff = neg[nkept - 1];
-                        std::vector<int64_t> result(nkept, -1);
-                        int64_t front = 0, back = nkept - 1;
-                        for (int64_t i = 0; i < np; ++i) {
-                            if (x[i] < cutoff) result[front++] = i;
-                            else if (x[i] == cutoff) { if (back >= front) result[back--] = i; }
-                        }
-                        for (int64_t idx : result) if (idx >= 0) { x[idx] = 0.0; active[idx] = 1; }
-                        conjugateGrads(n, np, r, w, p, y, AtWd, e0sq, active, x, wk, st);
-                    }
-                }
-                int64_t min_i = -1; double min_xi = -1.0;
-                for (int64_t i = 0; i < np; ++i)
-                    if (x[i] < 0.0) {
-                        const double xi = old_x[i] / (old_x[i] - x[i]);
-                        if (min_i == -1 || xi < min_xi) { min_i = i; min_xi = xi; }
-                    }
-                if (min_i == -1) break;
-                for (int64_t i = 0; i < np; ++i) if (!active[i]) old_x[i] = old_x[i] + min_xi * (x[i] - old_x[i]);
-                active[min_i] = 1;
-                x[min_i] = 0.0;
-            }
-            Ab(n, x, y.data(), wk);
-            Atx(n, y.data(), r.data(), wk);
-            int64_t min_i = -1; double min_grad = 1.0;
-            for (int64_t i = 0; i < np; ++i) {
-                double v = r[i] - AtWd[i];
-                r[i] = v * 2.0;
-                if (active[i]) { if (min_i == -1 || r[i] < min_grad) { min_i = i; min_grad = r[i]; } }
-            }
-            if (min_i == -1 || min_grad > -0.0000001) break;
-            active[min_i] = 0;
-        }
+        Work wk{std::vector<double>(np), std::vector<double>(np), std::vector<double>(n), std::vector<double>(n), std::vector<double>(n)};
+        activeConjugate(n, np, d, x, active, max_cg_iters > 0 ? std::min(np, max_cg_iters) : np, max_cg_calls, wk, st);
     }
+    if (active_out) std::copy(active.begin(), active.end(), active_out);
     if (stats) { stats[0] = st.cg_iters; stats[1] = st.cg_calls; stats[2] = st.outer; stats[3] = st.inner; }
     return 0;
 }

@@ -858,8 +858,7 @@ double normsq(const double* x, int64_t n) {
 struct CswStats { int64_t cg_iters = 0, cg_calls = 0, outer = 0, inner = 0; };
 // :769-831
 void conjugateGrads(int64_t ntax, int64_t npairs, double* r, double* w, double* p, double* y,
-                    const double* W, const double* b, const uint8_t* active, double* x, CswStats& st) {
-    int64_t kmax = ntax * (ntax - 1) / 2;
+                    const double* W, const double* b, const uint8_t* active, double* x, int64_t kmax, CswStats& st) {
     st.cg_calls++;
     calcAb(ntax, x, y);
     for (int64_t k = 0; k < npairs; k++) y[k] = W[k] * y[k];
@@ -905,27 +904,32 @@ bool worstIndices(const double* x, int64_t n, double propKept, std::vector<int64
     }
     return true;
 }
-// :359-557 (diagnostic prints dropped)
-void activeConjugate(int64_t ntax, int64_t npairs, const double* d, const double* W, double* x, CswStats& st) {
+// :359-557 (diagnostic prints dropped).  kmax: iteration cap of every CG call (npairs in the reference, :774);
+// max_cg_calls > 0: return right after that many CG calls (the budget of fnn_split_weights_budget).
+void activeConjugate(int64_t ntax, int64_t npairs, const double* d, const double* W, double* x, std::vector<uint8_t>& active,
+                     int64_t kmax, int64_t max_cg_calls, CswStats& st) {
     unconstrainedLS(ntax, d, x);
     bool all_positive = true;
     for (int64_t k = 0; k < npairs && all_positive; k++) if (x[k] < 0.0) all_positive = false;
     if (all_positive) return;
     std::vector<double> r(npairs), w(npairs), p(npairs), y(npairs), old_x(npairs, 1.0), AtWd(npairs);
-    std::vector<uint8_t> active(npairs, 0);
     for (int64_t k = 0; k < npairs; k++) y[k] = W[k] * d[k];
     calcAtx(ntax, y.data(), AtWd.data());
     bool first_pass = true;
     std::vector<int64_t> contract;
+    auto cg = [&]() {
+        conjugateGrads(ntax, npairs, r.data(), w.data(), p.data(), y.data(), W, AtWd.data(), active.data(), x, kmax, st);
+        return max_cg_calls > 0 && st.cg_calls >= max_cg_calls;   // budget spent
+    };
     while (true) {
         st.outer++;
         while (true) {
             st.inner++;
-            if (!first_pass) conjugateGrads(ntax, npairs, r.data(), w.data(), p.data(), y.data(), W, AtWd.data(), active.data(), x, st);
+            if (!first_pass && cg()) return;
             first_pass = false;
             if (worstIndices(x, npairs, 0.6, contract)) {
                 for (int64_t idx : contract) { x[idx] = 0.0; active[idx] = 1; }
-                conjugateGrads(ntax, npairs, r.data(), w.data(), p.data(), y.data(), W, AtWd.data(), active.data(), x, st);
+                if (cg()) return;
             }
             int64_t min_i = -1; double min_xi = -1.0;
             for (int64_t i = 0; i < npairs; i++) {
@@ -1020,15 +1024,21 @@ void oracle_atx(int64_t n, const double* d, double* p) { calcAtx(n, d, p); }
 void oracle_ab(int64_t n, const double* b, double* d) { calcAb(n, b, d); }
 
 // CircularSplitWeights.getWeights (:162-189) with var="ols" (W == 1), constrained.
-// d_pos: distances already in circular-position order (oracle_setup_d).
-int oracle_split_weights(int64_t n, const double* d_pos, double* x, int constrained, int64_t* stats /*[4]*/) {
+// d_pos: distances already in circular-position order (oracle_setup_d).  max_cg_iters / max_cg_calls: the budget of
+// fnn_split_weights_budget (include/fastnn.h), 0 = none.  active_out (optional, npairs bytes): 1 = split held at zero by the
+// active set when the solver returned.
+int oracle_split_weights(int64_t n, const double* d_pos, double* x, int constrained, int64_t* stats /*[4]*/, int64_t max_cg_iters,
+                         int64_t max_cg_calls, uint8_t* active_out) {
     int64_t npairs = n * (n - 1) / 2;
     CswStats st;
+    std::vector<uint8_t> active(npairs, 0);
     if (!constrained) unconstrainedLS(n, d_pos, x);
     else {
         std::vector<double> W(npairs, 1.0);   // v filled 1.0, W = 1/v (:172-177, :213-236)
-        activeConjugate(n, npairs, d_pos, W.data(), x, st);
+        activeConjugate(n, npairs, d_pos, W.data(), x, active, max_cg_iters > 0 ? std::min(npairs, max_cg_iters) : npairs,
+                        max_cg_calls, st);
     }
+    if (active_out) std::copy(active.begin(), active.end(), active_out);
     if (stats) { stats[0] = st.cg_iters; stats[1] = st.cg_calls; stats[2] = st.outer; stats[3] = st.inner; }
     return 0;
 }
