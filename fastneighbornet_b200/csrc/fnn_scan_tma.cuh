@@ -69,7 +69,7 @@ __device__ __forceinline__ double2 lds2(const double* p) { return *reinterpret_c
 // Interior evaluators: "filter, then verify".  The hot loop evaluates a role-free approximation
 // q~ = fma(c-2, Dpq~, -Sx[row]) - Sx[col] (fixed summation order, FMA allowed) and only tests
 // q~ <= best + delta, where delta bounds |q~ - q| for the exactly rounded, role-ordered q of the
-// reference (delta = 16*2^-53 * (3c+2) * max|D|, DESIGN.md §4).  Groups that pass are re-walked
+// reference (delta = 16*2^-53 * (3c+2) * max|D| + (c+2) * 2^-1074, DESIGN.md §4.1).  Groups that pass are re-walked
 // with the exact arithmetic and the (Q, i, j) key, so the result is bit-identical to evaluating
 // every entry exactly; on non-degenerate data the verify branch is taken a handful of times.
 __device__ __forceinline__ void exact1(double e, const RowData r, double cm2, double cS, int cP, double& bq,
@@ -202,8 +202,16 @@ k_scan_tma(const __grid_constant__ CUtensorMap tmap, const double* __restrict__ 
 
     double bq = INFINITY;
     unsigned long long bk = ~0ull;
-    // filter slack: bounds the rounding difference between the role-free q~ and the exact q
-    const double delta = 16.0 * 1.1102230246251565e-16 * (3.0 * (double)st->c + 2.0) * st->Dmax;
+    // filter slack: bounds the rounding difference between the role-free q~ and the exact q.  Every rounding is
+    // fl(x) = x(1+e) + h with |e| <= 2^-53 and |h| <= 2^-1075, h != 0 only for a product (or fma) whose result is below
+    // 2^-1022 (a sum or difference that lands there is exact).  The relative parts give the first term: every value is
+    // <= (c-2)*max|D| + 2c*max|D| and passes through <= 6 roundings in either form.  The absolute parts: the reference
+    // rounds Dpq (the *0.5 / *0.25 of a pair mean; its error is then multiplied by c-2) and (c-2)*Dpq, the role-free
+    // form rounds its fma once, and the product below may lose one more on underflow: <= (c+1) * 2^-1075, which
+    // (c+2) * 2^-1074 covers twice over.  For distances in the normal range that term is far below one ulp of delta
+    // and changes nothing.
+    const double delta = 16.0 * 1.1102230246251565e-16 * (3.0 * (double)st->c + 2.0) * st->Dmax
+                       + ((double)st->c + 2.0) * 4.9406564584124654e-324;
     double bqd = INFINITY;
 
     if (tid >= CONSUMERS) {

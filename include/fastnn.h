@@ -89,7 +89,10 @@ int fnn_device_count(void);
 /* ---- context API (device-resident matrix; used by bench `value` and by tests) ---------- */
 int fnn_ctx_create(const fnn_opts* o, int64_t n, fnn_ctx** out);
 void fnn_ctx_destroy(fnn_ctx* c);
-/* upload an n*n row-major symmetric zero-diagonal host matrix (the Java double[][] D of FastNN.java:307-312) */
+/* upload an n*n row-major symmetric zero-diagonal host matrix (the Java double[][] D of FastNN.java:307-312).
+ * Verified domain of the ordering (bit-identical to the reference's arithmetic): finite, non-negative entries, subnormal
+ * values included, with max|D| small enough that 3n*max|D| stays finite.  Negative or non-finite entries are outside
+ * the contract. */
 int fnn_ctx_load_host(fnn_ctx* c, const double* D_rowmajor);
 /* multi-GPU upload without replicating the PCIe traffic: upload only rows [row0, row0+nrows) (nrows*n doubles, row-major);
  * the host layer moves the row blocks between the ranks over NVLink (e.g. torch.distributed.broadcast on the matrix of
@@ -128,7 +131,8 @@ int fnn_ctx_connect(fnn_ctx* c, int32_t rank, int32_t world, const void* handles
 /* ---- one-shot seams ----------------------------------------------------------------- */
 /* B1: replaces `new NeighborNetX(D, n, ...).runNeighborNet()`.  Exactly one of D_rowmajor
  * (host, n*n) or phylip_path must be non-NULL.  n<=3 returns the identity ordering
- * (NetMakerOriginal.java:133-140). */
+ * (NetMakerOriginal.java:133-140).  The matrix must be symmetric with a zero diagonal; the verified domain is that of
+ * fnn_ctx_load_host (finite, non-negative, subnormal values included, 3n*max|D| finite). */
 int fnn_order(const fnn_opts* o, const double* D_rowmajor, const char* phylip_path, int64_t n, int32_t* ordering_out);
 /* fnn_order keeps its last context (device buffers, tensor map, instantiated CUDA graph) for the next call with the same n
  * and options; this releases it (the JNI shim calls it from JNI_OnUnload). */

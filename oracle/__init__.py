@@ -34,7 +34,8 @@ def lib():
         c_ip = ctypes.POINTER(ctypes.c_int32)
         c_lp = ctypes.POINTER(ctypes.c_int64)
         L.oracle_order.argtypes = [ctypes.c_int, ctypes.c_int64, c_dp, ctypes.c_int64, ctypes.c_int, ctypes.c_int,
-                                   ctypes.c_int, c_ip, c_dp, ctypes.c_int64, c_lp, c_lp, ctypes.c_int, c_dp]
+                                   ctypes.c_int, c_ip, c_dp, ctypes.c_int64, c_lp, c_lp, ctypes.c_int, c_dp,
+                                   ctypes.c_int64]
         L.oracle_order.restype = ctypes.c_int
         L.oracle_rowsums.argtypes = [ctypes.c_int64, c_dp, c_dp]
         L.oracle_setup_d.argtypes = [ctypes.c_int64, c_ip, c_dp, c_dp]
@@ -72,8 +73,10 @@ def _bp(a):
     return a.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
 
 
-def order(D, mode="canonical", seed=12345, mult=5, additive=False, fallback=1024, want_trace=True, threads=1):
-    """Returns (ordering[n+1] int32, trace[k,8] float64, counters dict).  D is copied."""
+def order(D, mode="canonical", seed=12345, mult=5, additive=False, fallback=1024, want_trace=True, threads=1, max_iters=0):
+    """Returns (ordering[n+1] int32, trace[k,8] float64, counters dict).  D is copied.
+    max_iters = K > 0: stop after K agglomeration iterations; the trace is then the first K rows of the full trace and the
+    ordering is undefined (all zeros).  0 = no limit."""
     n = D.shape[0]
     Dc = np.array(D, dtype=np.float64, order="C", copy=True)
     ordering = np.zeros(n + 1, dtype=np.int32)
@@ -83,7 +86,7 @@ def order(D, mode="canonical", seed=12345, mult=5, additive=False, fallback=1024
     cnt = np.zeros(2, dtype=np.int64)
     ab = np.zeros(1, dtype=np.float64)
     rc = lib().oracle_order(MODES[mode], n, _dp(Dc), seed, mult, int(additive), fallback, _ip(ordering),
-                            _dp(trace) if want_trace else None, max_trace, _lp(ntr), _lp(cnt), int(threads), _dp(ab))
+                            _dp(trace) if want_trace else None, max_trace, _lp(ntr), _lp(cnt), int(threads), _dp(ab), int(max_iters))
     if rc != 0:
         raise RuntimeError(f"oracle_order rc={rc}")
     return ordering, trace[: int(ntr[0])], {"pair_evals": int(cnt[0]), "npe_would_fire": int(cnt[1]), "D_final": Dc,

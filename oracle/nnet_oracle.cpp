@@ -161,6 +161,8 @@ struct Engine {
     std::unique_ptr<SlicePool> pool;
     std::vector<TraceRow>* trace = nullptr;
     int status = 0;
+    int64_t max_iters = 0;       // >0: stop after this many agglomeration iterations (the ordering is then undefined)
+    bool stopped = false;
 
     inline double& d(int a, int b) { return D[nd[a].dist * n + nd[b].dist]; }
 
@@ -697,7 +699,8 @@ struct Engine {
     // NetMakerOriginal.java:331-395
     int agglomNodes(int num_nodes) {
         int num_active = num_nodes, num_clusters = num_nodes;
-        while (num_active > 3) {
+        for (int64_t iter = 0; num_active > 3; ++iter) {
+            if (max_iters > 0 && iter >= max_iters) { stopped = true; break; }
             if (num_active == 4 && num_clusters == 2) {
                 int p = act[0];
                 int q = (nd[p].nbr != act[1]) ? act[1] : act[2];
@@ -773,6 +776,7 @@ struct Engine {
         initialize((int)n);
         agglomNodes((int)n);
         if (status != 0) return status;
+        if (stopped) { for (int64_t i = 0; i <= n; ++i) ordering[i] = 0; return 0; }
         expandNodes(ordering);
         return 0;
     }
@@ -974,11 +978,15 @@ void oracle_set_relaxed_sm(int on) { g_use_relaxed_sm = on; }
 
 // Ordering.  D is n*n row-major and is mutated in place (like the Java double[][]).
 // trace_out: optional [max_trace][8] doubles (m,c,cx,cy,x,y,kind,best); returns rows in *n_trace.
+// max_iters > 0: stop after that many agglomeration iterations and return the trace so far (a prefix of the full trace);
+// the ordering is then all zeros.  0 = run to the end.
 int oracle_order(int mode, int64_t n, double* D, int64_t seed, int mult, int additive, int fallback,
                  int32_t* ordering, double* trace_out, int64_t max_trace, int64_t* n_trace,
-                 int64_t* counters /* [0]=pair_evals [1]=npe_would_fire */, int threads, double* alg_bytes) {
+                 int64_t* counters /* [0]=pair_evals [1]=npe_would_fire */, int threads, double* alg_bytes,
+                 int64_t max_iters) {
     Engine e;
     e.n = n; e.D = D; e.mode = mode; e.mult = mult; e.additive = additive != 0; e.fallback = fallback;
+    e.max_iters = max_iters;
     e.rng = JavaRandom(seed);
     e.threads = threads < 1 ? 1 : threads;
     std::vector<TraceRow> tr;

@@ -12,6 +12,7 @@ import struct
 from fractions import Fraction
 
 import numpy as np
+import pytest
 
 from oracle import pyref
 
@@ -310,18 +311,43 @@ def _rn(fr):
     return float(fr)   # Fraction -> nearest double, ties to even
 
 
+def _scan_slack(c, dmax):
+    """The filter slack of k_scan_tma, in the kernel's operation order (fnn_scan_tma.cuh: delta)."""
+    return 16.0 * 1.1102230246251565e-16 * (3.0 * float(c) + 2.0) * dmax + (float(c) + 2.0) * 2.0**-1074
+
+
+def _scale_of(cls, rng):
+    """max|D| of one scale class: 'normal' 10^U(-3, 3); 'sub' an integer multiple of 2^-1074 up to 2^-1000 (subnormal and
+    just above); 'band' 2^U(-1074, -1022), the subnormal range itself; 'edge' an integer multiple of 2^-1074 below 64."""
+    if cls == "normal":
+        return float(10.0 ** rng.uniform(-3, 3))
+    if cls == "sub":
+        return math.ldexp(float(rng.integers(1, 2**52)), int(rng.integers(-1074, -1052)))
+    if cls == "band":
+        return max(float(2.0 ** rng.uniform(-1074, -1022)), 2.0**-1074)
+    return math.ldexp(float(rng.integers(1, 64)), -1074)
+
+
 def test_scan_filter_slack_bounds_the_rounding_difference():
-    """delta = 16 * 2^-53 * (3c + 2) * max|D| must dominate |q~ - q| for every role order (fnn_scan_tma.cuh)."""
-    rng = np.random.default_rng(4)
+    """delta = 16 * 2^-53 * (3c + 2) * max|D| + (c + 2) * 2^-1074 must dominate |q~ - q| for every role order
+    (fnn_scan_tma.cuh), for max|D| from the normal range down to a few subnormal ulps.  Below 2^-1022 a rounded product
+    carries an absolute error of up to 2^-1075 that no relative term covers, and the reference's rounding of Dpq is then
+    multiplied by c - 2: the second term of delta."""
+    for cls in ("normal", "sub", "band", "edge"):
+        _scan_slack_case(cls)
+
+
+def _scan_slack_case(cls):
+    rng = np.random.default_rng({"normal": 4, "sub": 5, "band": 6, "edge": 7}[cls])
     worst = 0.0
     for trial in range(4000):
-        c = int(rng.integers(3, 200000))
-        dmax = float(10.0 ** rng.uniform(-3, 3))
+        c = int(rng.integers(3, 200000)) if trial % 4 else int(rng.integers(3, 40))
+        dmax = _scale_of(cls, rng)
         a, b, cc, d = (float(v) for v in rng.random(4) * dmax)
         # cluster row sums are sums of <= c cluster distances, each <= dmax
         sp, sq = (float(v) for v in rng.random(2) * c * dmax)
         cm2 = float(c) - 2.0
-        delta = 16.0 * 2.0**-53 * (3.0 * c + 2.0) * dmax
+        delta = _scan_slack(c, dmax)
         kind = trial % 3
         exact = []
         if kind == 0:      # pair x pair: both role orders of the 4-term mean and of the subtractions
@@ -339,8 +365,8 @@ def test_scan_filter_slack_bounds_the_rounding_difference():
             approx = _rn(Fraction(cm2) * Fraction(a) - Fraction(sp)) - sq
         for q in exact:
             worst = max(worst, abs(approx - q) / delta)
-            assert abs(approx - q) <= delta, (trial, kind, approx, q, delta)
-    assert worst < 0.5   # the bound has slack to spare
+            assert abs(approx - q) <= delta, (cls, trial, kind, c, dmax, approx, q, delta)
+    assert worst < 0.5, (cls, worst)   # the bound has slack to spare
 
 
 # ------------------------------------------------------------------ certified 4-candidate pick model (csrc/fnn_order.cu: k_pick)
@@ -385,9 +411,20 @@ def _certificate(m, f, d, terms, present):
     return (ks if cert else None), kx
 
 
+# binary exponents by which the certificate's model inputs are scaled: none, then down through the subnormal range, where
+# products carry an absolute rounding error and the bounds themselves underflow
+PICK_SHIFTS = (0, -1000, -1022, -1040, -1060, -1074)
+
+
 def test_summation_order_bound_of_the_certificate():
     """|left-to-right sum - any other order| <= (2m+256) * 2^-53 * sum|a| : the E of the certificate, on adversarial inputs
-    (wide magnitude ranges, alternating signs, sorted either way)."""
+    (wide magnitude ranges, alternating signs, sorted either way), scaled by 2^shift down to the subnormal range (there
+    every sum whose running value stays below 2^-1022 is exact, and a bound that underflows must still hold)."""
+    for shift in PICK_SHIFTS:
+        _summation_order_case(shift)
+
+
+def _summation_order_case(shift):
     rng = np.random.default_rng(5)
     for m in (7, 100, 3001, 20000):
         for kind in range(6):
@@ -402,6 +439,7 @@ def test_summation_order_bound_of_the_certificate():
                 a = a * np.where(rng.random(m) < 0.5, -1.0, 1.0) * 10.0 ** rng.integers(-3, 3, m)
             elif kind == 5:
                 a = np.concatenate([[1e16], rng.random(m - 1)])
+            a = np.ldexp(a, shift)
             seq = _seq_sum(a)
             bound = (2.0 * m + 256.0) * U53 * float(np.sum(np.abs(a)))
             for other in (float(np.sum(a)), float(np.sum(a[::-1])), float(np.sum(rng.permutation(a))), math.fsum(a),
@@ -411,7 +449,13 @@ def test_summation_order_bound_of_the_certificate():
 
 def test_certified_pick_never_disagrees_with_the_exact_sums():
     """Whenever the certificate accepts, the candidate it names is the one the reference's exact left-to-right sums pick;
-    on exact ties and near-ties it must refuse.  Random, tie and near-tie instances."""
+    on exact ties and near-ties it must refuse.  Random, tie and near-tie instances, with terms and distances scaled by
+    2^shift down to the subnormal range."""
+    for shift in PICK_SHIFTS:
+        _certified_pick_case(shift)
+
+
+def _certified_pick_case(shift):
     rng = np.random.default_rng(11)
     accepted = refused = 0
     for trial in range(400):
@@ -426,8 +470,8 @@ def test_certified_pick_never_disagrees_with_the_exact_sums():
             base[1, 0] = np.nextafter(base[1, 0], 2.0)
             base[3, -1] = np.nextafter(base[3, -1], 0.0)
         w = np.where(rng.random(m) < 0.5, 1.0, 0.5)
-        terms = [base[r] * w for r in range(4)]
-        d = rng.random(4) if mode in (0, 3) else np.full(4, 0.5)
+        terms = [np.ldexp(base[r], shift) * w for r in range(4)]
+        d = np.ldexp(rng.random(4) if mode in (0, 3) else np.full(4, 0.5), shift)
         present = (True, bool(rng.integers(0, 2)) or mode != 0, bool(rng.integers(0, 2)) or mode != 0, False)
         present = present[:3] + (present[1] and present[2],)
         ks, kx = _certificate(m, f, d, terms, present)
@@ -438,4 +482,4 @@ def test_certified_pick_never_disagrees_with_the_exact_sums():
             assert ks == kx, (trial, mode, ks, kx)
         if mode == 1 and sum(present) > 1:
             assert ks is None   # exact ties are never certified
-    assert accepted > 100 and refused > 100
+    assert accepted > 100 and refused > 100, (shift, accepted, refused)

@@ -128,6 +128,23 @@ def test_iteration_counts_and_kinds():
     assert info["pair_evals"] == sum(int(c) * (int(c) - 1) // 2 for c in tr[tr[:, 6] != 5][:, 1])
 
 
+@pytest.mark.parametrize("mode,fb,additive", [("canonical", 1024, False), ("relaxed", 8, False), ("relaxed", 8, True),
+                                              ("random_n", 8, False), ("random_nlogn", 8, False), ("random_logn", 8, False)])
+def test_iteration_budget_gives_a_prefix_of_the_trace(mode, fb, additive):
+    """oracle.order(max_iters=K) stops after K agglomeration iterations: its trace is the first K rows of the full trace (K
+    below, at and beyond the full length), whatever the mode, the thread count or the matrix."""
+    for D in (tree_matrix(60, 3, 0.05), integer_matrix(45, 4, hi=4)):
+        o_full, t_full, _ = oracle.order(D, mode=mode, seed=21, fallback=fb, additive=additive)
+        k_full = t_full.shape[0]
+        for K in (1, 2, 7, k_full // 2, k_full - 1, k_full, k_full + 5):
+            for threads in (1, 3):
+                o, t, _ = oracle.order(D, mode=mode, seed=21, fallback=fb, additive=additive, threads=threads, max_iters=K)
+                assert t.shape == (min(K, k_full), 8)
+                assert (t == t_full[:K]).all()
+                if K >= k_full:
+                    assert (o == o_full).all()
+
+
 def test_threaded_canonical_equals_single_thread():
     D = tree_matrix(1300, 3, 0.05)
     o1, t1, _ = oracle.order(D, threads=1)
