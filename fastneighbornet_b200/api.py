@@ -61,7 +61,7 @@ ABI_SYMBOLS = [
     "fnn_ctx_trace", "fnn_ctx_stats", "fnn_ctx_matrix_ptr", "fnn_order", "fnn_rowsums", "fnn_seq_sum",
     "fnn_split_weights", "fnn_csw_matvec", "fnn_ctx_ipc_handle", "fnn_ctx_connect", "fnn_weighted_splits", "fnn_network",
     "fnn_phylip_taxa", "fnn_read_phylip", "fnn_write_nexus", "fnn_java_double_to_string", "fnn_release_cache",
-    "fnn_ctx_load_host_rows", "fnn_ctx_commit_load", "fnn_split_weights_budget",
+    "fnn_ctx_load_host_rows", "fnn_ctx_commit_load", "fnn_split_weights_budget", "fnn_ctx_strategy_record",
 ]
 
 
@@ -95,6 +95,8 @@ def lib():
         L.fnn_ctx_order.argtypes = [vp, ctypes.POINTER(ctypes.c_int32)]
         L.fnn_ctx_trace.argtypes = [vp, c_dp, ctypes.c_int64]
         L.fnn_ctx_trace.restype = ctypes.c_int64
+        L.fnn_ctx_strategy_record.argtypes = [vp, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64]
+        L.fnn_ctx_strategy_record.restype = ctypes.c_int64
         L.fnn_ctx_stats.argtypes = [vp, ctypes.POINTER(fnn_stats)]
         L.fnn_ctx_matrix_ptr.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(ctypes.c_int64)]
         L.fnn_ctx_ipc_handle.argtypes = [vp, ctypes.c_char_p]
@@ -280,6 +282,16 @@ class Context:
     def trace(self):
         rows = np.zeros((self.n + 8, 8), dtype=np.float64)
         k = lib().fnn_ctx_trace(self._h, _dp(rows), rows.shape[0])
+        if k < 0:
+            _check(int(k))
+        return rows[: int(k)]
+
+    def strategy_record(self):
+        """Per-iteration strategy record (fnn_ctx_strategy_record; needs record_trace=1): an (iterations, 4) int64 array,
+        Random: draws, rejected draws, remapped draws, digest; Relaxed: row scans, ties, look-aheads, digest.  Column 3 is a
+        uint64 digest stored as int64 (view it with .view(np.uint64))."""
+        rows = np.zeros((self.n + 8, 4), dtype=np.int64)
+        k = lib().fnn_ctx_strategy_record(self._h, rows.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), rows.shape[0])
         if k < 0:
             _check(int(k))
         return rows[: int(k)]

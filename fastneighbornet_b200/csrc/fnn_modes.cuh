@@ -9,6 +9,7 @@
 //           :88-126) and the -additive look-ahead (:280-466) it asks for.
 #pragma once
 #include "fnn_relaxed_sm.h"
+#include "fnn_record.h"
 
 namespace modes {
 
@@ -91,7 +92,7 @@ __device__ __forceinline__ long long random_search_amount(int mode, int mult, in
 
 __global__ void __launch_bounds__(THREADS, 1)
 k_random_walk(const int* __restrict__ pos, const int* __restrict__ p2s, DevState* st, int* __restrict__ nbrpos,
-              int2* __restrict__ pairs, WalkState* ws) {
+              int2* __restrict__ pairs, WalkState* ws, long long* __restrict__ record) {
     if (st->done || st->mode < 2 || st->m <= st->fallback) return;
     __shared__ unsigned long long Ap[24], Cp[24];
     __shared__ unsigned char wfun[THREADS / 32];
@@ -100,6 +101,7 @@ k_random_walk(const int* __restrict__ pos, const int* __restrict__ p2s, DevState
     __shared__ unsigned long long s_base;
     __shared__ int s_cur, s_exc;
     __shared__ long long s_count;
+    __shared__ long long s_rejected, s_remapped;   // strategy record (only when one is kept)
     const int m = st->m, P2 = st->P2, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const long long total = random_search_amount(st->mode, st->mult, m);
     if (tid == 0) tl_stamp(st, TL_SCAN0);
@@ -115,6 +117,7 @@ k_random_walk(const int* __restrict__ pos, const int* __restrict__ p2s, DevState
         s_cur = jr_next_int(rng, m);   // int i = myRandom.nextInt(num_active) (:134)
         s_base = rng;
         s_count = 0;
+        s_rejected = s_remapped = 0;
     }
     __syncthreads();   // also publishes nbrpos (block-local producer/consumer through global memory)
     __threadfence_block();
@@ -216,16 +219,21 @@ k_random_walk(const int* __restrict__ pos, const int* __restrict__ p2s, DevState
             if (exc < wlen) {   // replay the exceptional draw exactly
                 const int i = s_cur;
                 const int inb = nbrpos[i];
-                int j;
+                const unsigned long long one_step = (rng * JR_A + JR_C) & JR_MASK;
+                int j, j0;
                 if (inb >= 0) {
-                    j = jr_next_int(rng, m - 2);
+                    j = j0 = jr_next_int(rng, m - 2);
                     if (i == j && m - 1 == inb) j = m - 2;
                     else if (i == j && m - 1 != inb) j = m - 1;
                     else if (inb == j && m - 2 == i) j = m - 1;
                     else if (inb == j && m - 2 != i) j = m - 2;
                 } else {
-                    j = jr_next_int(rng, m - 1);
+                    j = j0 = jr_next_int(rng, m - 1);
                     if (i == j) j = m - 1;
+                }
+                if (record) {   // the exception was a rejection (nextInt took more than one LCG step), a remap, or both
+                    s_rejected += rng != one_step;
+                    s_remapped += j != j0;   // every remap target lies outside nextInt's range, so a remap always changes j
                 }
                 pairs[count + exc] = make_int2(i, j);
                 s_cur = j;
@@ -240,13 +248,18 @@ k_random_walk(const int* __restrict__ pos, const int* __restrict__ p2s, DevState
         st->rng = s_base;
         ws->count = s_count;
         ws->total = total;
+        if (record) {   // k_random_eval adds the digest (column 3)
+            long long* row = record + rec::COLS * (int64_t)st->iter;
+            row[0] = s_count; row[1] = s_rejected; row[2] = s_remapped;
+        }
     }
 }
 
 // Q for every committed pair, min-loc on (Q, draw index); the last block reduces the partials
 __global__ void __launch_bounds__(256)
 k_random_eval(const double* __restrict__ D, int64_t ld, const double* __restrict__ Sx, const int* __restrict__ p2s,
-              DevState* st, const int2* __restrict__ pairs, const WalkState* ws, Partial* partials, unsigned int* ticket) {
+              DevState* st, const int2* __restrict__ pairs, const WalkState* ws, Partial* partials, unsigned int* ticket,
+              long long* __restrict__ record) {
     if (st->done || st->mode < 2 || st->m <= st->fallback) return;
     __shared__ double wq[8];
     __shared__ unsigned long long wk[8];
@@ -257,8 +270,10 @@ k_random_eval(const double* __restrict__ D, int64_t ld, const double* __restrict
     double bq = INFINITY;
     unsigned long long bk = ~0ull;
     unsigned long long abytes = 0;   // SURVEY 8(d) K9: 8*(1|2|4) + 16 bytes per sample
+    unsigned long long digest = 0;   // strategy record: this thread's share of the draws' digest (fnn_record.h)
     for (long long k = (long long)blockIdx.x * blockDim.x + tid; k < total; k += (long long)gridDim.x * blockDim.x) {
         const int2 pr = pairs[k];
+        if (record) digest += rec::draw_term(k, pr.x, pr.y);
         const int sp = p2s[pr.x], sq = p2s[pr.y];
         abytes += 8ull * (unsigned)((1 + (sp < P2)) * (1 + (sq < P2))) + 16ull;
         const double q = (cm2 * dpq_roles(D, ld, sp, sq, P2) - Sx[sp]) - Sx[sq];
@@ -274,6 +289,11 @@ k_random_eval(const double* __restrict__ D, int64_t ld, const double* __restrict
     }
     for (int off = 16; off > 0; off >>= 1) abytes += __shfl_down_sync(0xffffffffu, abytes, off);
     if ((tid & 31) == 0) { wq[tid >> 5] = bq; wk[tid >> 5] = bk; if (abytes) atomicAdd(&st->strat_bytes, abytes); }
+    if (record) {   // a sum mod 2^64: the order in which the warps add their shares does not matter
+        for (int off = 16; off > 0; off >>= 1) digest += __shfl_down_sync(0xffffffffu, digest, off);
+        if ((tid & 31) == 0 && digest)
+            atomicAdd(reinterpret_cast<unsigned long long*>(record + rec::COLS * (int64_t)st->iter + 3), digest);
+    }
     __syncthreads();
     if (tid == 0) {
         for (int w = 1; w < 8; ++w) take(wq[w], wk[w]);
@@ -499,12 +519,14 @@ struct DevNodeView {
 
 __global__ void __launch_bounds__(THREADS, 1)
 k_relaxed_select(const double* __restrict__ D, int64_t ld, const double* __restrict__ Sx, const int* __restrict__ id,
-                 const int* __restrict__ pos, const int* __restrict__ p2s, DevState* st, relaxed::Machine* Mg, int ntax) {
+                 const int* __restrict__ pos, const int* __restrict__ p2s, DevState* st, relaxed::Machine* Mg, int ntax,
+                 long long* __restrict__ record) {
     if (st->done || st->mode != 1 || st->m <= st->fallback) return;
     extern __shared__ unsigned char smem_raw[];
     xsum::Smem* xs = reinterpret_cast<xsum::Smem*>(smem_raw);
     __shared__ relaxed::Machine M;
     __shared__ int req, look_accept;
+    __shared__ long long s_rec[rec::COLS];   // strategy record (only when one is kept): scans, ties, look-aheads, digest
     const int m = st->m, c = st->c, P2 = st->P2, tid = threadIdx.x;
     const double cm2 = (double)c - 2.0;
     const DevNodeView nv{id, pos, p2s, m, P2};
@@ -513,6 +535,7 @@ k_relaxed_select(const double* __restrict__ D, int64_t ld, const double* __restr
         M = *Mg;
         relaxed::begin_call(M, ntax);
         look_accept = 0;
+        for (int k = 0; k < rec::COLS; ++k) s_rec[k] = 0;
     }
     __syncthreads();
     while (true) {
@@ -526,12 +549,20 @@ k_relaxed_select(const double* __restrict__ D, int64_t ld, const double* __restr
                 // SURVEY 8(d) K7: a row scan reads the row (two rows if p is paired) and Sx
                 st->strat_bytes += 8ull * (unsigned long long)m * (unsigned)(1 + (p2s[M.req_pos] < P2)) + 8ull * (unsigned long long)m;
                 st->strat_units += 1;
+                if (record) {   // block_rowmin has sorted the ties and written them (visible after its last barrier)
+                    const int s = (int)s_rec[0];
+                    unsigned long long dg = rec::scan_term(s, M.req_pos, -1, 0);
+                    for (int r = 0; r < cnt; ++r) dg += rec::scan_term(s, M.req_pos, r, M.tiepool[M.tie_used + r]);
+                    s_rec[0] += 1;
+                    if (cnt > 0) s_rec[1] += cnt;
+                    s_rec[3] = (long long)((unsigned long long)s_rec[3] + dg);
+                }
                 if (cnt < 0) M.error = 3;
                 else relaxed::commit_scan(M, cnt);
             }
         } else {
             const bool acc = block_lookahead(D, ld, Sx, p2s, m, c, P2, M.cx_pos, M.cy_pos, M.look_test_pos, xs);
-            if (tid == 0) look_accept = acc ? 1 : 0;
+            if (tid == 0) { look_accept = acc ? 1 : 0; s_rec[2] += 1; }
         }
         __threadfence_block();
         __syncthreads();
@@ -542,6 +573,8 @@ k_relaxed_select(const double* __restrict__ D, int64_t ld, const double* __restr
         st->cy_pos = M.cy_pos;
         if (M.error || M.cx_pos < 0 || M.cy_pos < 0) { st->error = 10 + M.error; st->done = 1; st->skip = 1; }
         *Mg = M;
+        if (record)
+            for (int k = 0; k < rec::COLS; ++k) record[rec::COLS * (int64_t)st->iter + k] = s_rec[k];
         tl_stamp(st, TL_SCAN1);
     }
 }

@@ -44,6 +44,7 @@
 #include "fastnn.h"
 #include "fnn_common.h"
 #include "fnn_relaxed_sm.h"
+#include "fnn_record.h"
 
 namespace {
 
@@ -953,12 +954,14 @@ struct fnn_ctx {
     unsigned int* walk_ticket = nullptr;
     int64_t rxs_ld = 0;
     double* trace = nullptr;
+    long long* record = nullptr;      // per-iteration strategy record (fnn_record.h), kept with the trace
     int *id = nullptr, *pos = nullptr, *p2s = nullptr, *amalg = nullptr;
     DevState* st = nullptr;
-    Partial* partials = nullptr;
+    Partial* partials = nullptr;      // per-block partial min-locs of k_scan_tma and k_random_eval
+    int partials_cap = 0;             // ... and their number: no grid that writes them may be larger
     double* rx_part = nullptr;        // per-block partial ComputeRx sums of k_rx_stage
     Partial* patch_part = nullptr;    // per-block partial min-locs of k_patch
-    int scan_grid = 0, row_grid = 0;
+    int scan_grid = 0, row_grid = 0, eval_grid = 0;
     // u.Sx chain + new-cluster patch on a forked branch, concurrent with the next scan (which then leaves one SM to it)
     size_t chain_smem = 0;            // k_chain + k_patch: exact-summation workspace + (if it fits) the staged chain
     int chain_stage_cap = 0;          // elements of the chain that fit in shared memory (0: read from global)
@@ -1028,7 +1031,7 @@ extern "C" void fnn_ctx_destroy(fnn_ctx* c) {
     if (c->graph_strategy) cudaGraphExecDestroy(c->graph_strategy);
     cudaFree(c->rl_machine); cudaFree(c->rl_rowPerm); cudaFree(c->rl_epoch); cudaFree(c->rl_clist); cudaFree(c->rl_loff);
     cudaFree(c->rl_lcnt); cudaFree(c->rl_lme); cudaFree(c->rl_tie); cudaFree(c->rl_mymin);
-    cudaFree(c->D); cudaFree(c->Sx); cudaFree(c->scratch); cudaFree(c->stage); cudaFree(c->rxs); cudaFree(c->trace);
+    cudaFree(c->D); cudaFree(c->Sx); cudaFree(c->scratch); cudaFree(c->stage); cudaFree(c->rxs); cudaFree(c->trace); cudaFree(c->record);
     for (int r = 0; r < MAX_WORLD; ++r) if (c->opened[r]) cudaIpcCloseMemHandle(c->opened[r]);
     cudaFree(c->mail); cudaFree(c->peers);
     cudaFree(c->nbrpos); cudaFree(c->pairs); cudaFree(c->walk); cudaFree(c->walk_ticket);
@@ -1050,6 +1053,9 @@ extern "C" int fnn_ctx_create(const fnn_opts* o, int64_t n, fnn_ctx** out) {
     if (!o) { fnn_default_opts(&d); o = &d; }
     if (n > 2000000) { fnn::set_error("n too large"); return FNN_E_ARG; }
     if (o->mode < 0 || o->mode > FNN_RANDOM_LOGN) { fnn::set_error("unknown mode %d", o->mode); return FNN_E_ARG; }
+    // a Random mode draws mult * amount pairs per iteration (NeighborNetRandom.java:31-48); with none the reference has no
+    // Cx (NullPointerException) and k_random_eval would have no pair to select
+    if (o->mode >= FNN_RANDOM_N && o->mult < 1) { fnn::set_error("mult %d: a Random mode needs mult >= 1", o->mult); return FNN_E_ARG; }
 
     int rc = ensure_device(o);
     if (rc) return rc;
@@ -1101,10 +1107,15 @@ static int ctx_build(fnn_ctx* c, const fnn_opts* o, int64_t n) {
     c->force_exact = (o->reserved[5] & 2) ? 1 : 0;
     c->scan_grid = c->sms - (c->overlap ? 1 : 0);
     c->row_grid = std::max<int>(1, std::min<int64_t>((n + 255) / 256, std::min(c->sms * 4, RX_BLOCKS_MAX)));
-    FNN_ALLOC(c->partials, sizeof(Partial) * c->sms);
+    c->eval_grid = c->sms * 2;
+    c->partials_cap = std::max(c->scan_grid, c->eval_grid);
+    FNN_ALLOC(c->partials, sizeof(Partial) * c->partials_cap);
     FNN_ALLOC(c->rx_part, sizeof(double) * 8 * RX_BLOCKS_MAX);
     FNN_ALLOC(c->patch_part, sizeof(Partial) * PATCH_BLOCKS);
-    if (o->record_trace) FNN_ALLOC(c->trace, sizeof(double) * 8 * (n + 8));
+    if (o->record_trace) {
+        FNN_ALLOC(c->trace, sizeof(double) * 8 * (n + 8));
+        FNN_ALLOC(c->record, sizeof(long long) * rec::COLS * (n + 8));
+    }
     if (o->mode == FNN_RELAXED) {
         c->rl_max_lists = (int)(2 * n + 16); c->rl_tie_cap = (int)(16 * n + 65536); c->rl_mymin_cap = (int)(8 * n + 65536);
         FNN_ALLOC(c->rl_machine, sizeof(relaxed::Machine));
@@ -1224,8 +1235,18 @@ extern "C" int fnn_ctx_matrix_ptr(fnn_ctx* c, double** dptr, int64_t* ld) {
 
 static_assert(PICK_THREADS == xsum::THREADS, "exact-sum block size");
 
-static inline void launch_scan(fnn_ctx* c) {
+// Every block of k_scan_tma and k_random_eval writes partials[blockIdx.x] and the last one reads them all: a grid larger than
+// the allocation would write past its end without any fault to show it.
+static inline int check_partials(fnn_ctx* c, int grid, const char* kernel) {
+    if (grid <= c->partials_cap) return FNN_OK;
+    fnn::set_error("%s: grid of %d blocks, but partials holds %d", kernel, grid, c->partials_cap);
+    return FNN_E_STATE;
+}
+
+static inline int launch_scan(fnn_ctx* c) {
+    if (int rc = check_partials(c, c->scan_grid, "k_scan_tma")) return rc;
     tma::k_scan_tma<<<c->scan_grid, tma::THREADS, tma::SMEM_BYTES, c->stream>>>(c->tmap, c->Sx, c->pos, c->st, c->partials, c->peers);
+    return FNN_OK;
 }
 
 // 2-D tiled tensor map over the n x ld matrix: box = 256 columns x 8 rows, no swizzle, zero OOB fill
@@ -1250,16 +1271,18 @@ static int make_tensor_map(fnn_ctx* c) {
 }
 // everything of an iteration after the scan.  The previous iteration's k_chain + k_patch (forked branch) joins here: the
 // strategy kernels, the selection merge and the update all need the new cluster's exact Sx.
-static inline void launch_rest(fnn_ctx* c) {
+static inline int launch_rest(fnn_ctx* c) {
+    if (c->o.mode >= FNN_RANDOM_N)
+        if (int rc = check_partials(c, c->eval_grid, "k_random_eval")) return rc;
     if (c->join_pending) { cudaStreamWaitEvent(c->stream, c->ev_join, 0); c->join_pending = false; }
     if (c->o.mode >= FNN_RANDOM_N) {
-        modes::k_random_walk<<<1, modes::THREADS, 0, c->stream>>>(c->pos, c->p2s, c->st, c->nbrpos, c->pairs, c->walk);
-        modes::k_random_eval<<<c->sms * 2, 256, 0, c->stream>>>(c->D, c->ld, c->Sx, c->p2s, c->st, c->pairs, c->walk, c->partials,
-                                                                c->walk_ticket);
+        modes::k_random_walk<<<1, modes::THREADS, 0, c->stream>>>(c->pos, c->p2s, c->st, c->nbrpos, c->pairs, c->walk, c->record);
+        modes::k_random_eval<<<c->eval_grid, 256, 0, c->stream>>>(c->D, c->ld, c->Sx, c->p2s, c->st, c->pairs, c->walk, c->partials,
+                                                                  c->walk_ticket, c->record);
     }
     if (c->o.mode == FNN_RELAXED)
         modes::k_relaxed_select<<<1, modes::THREADS, sizeof(xsum::Smem), c->stream>>>(c->D, c->ld, c->Sx, c->id, c->pos, c->p2s, c->st,
-                                                                                     c->rl_machine, (int)c->n);
+                                                                                     c->rl_machine, (int)c->n, c->record);
     k_rx_stage<<<c->row_grid, 256, 0, c->stream>>>(c->D, c->ld, c->id, c->pos, c->p2s, c->st, c->mail, c->rxs, c->rxs_ld, c->rx_part);
     k_pick<<<1, PICK_THREADS, PICK_SMEM, c->stream>>>(c->D, c->ld, c->Sx, c->id, c->pos, c->p2s, c->st, c->amalg, c->trace,
                                                     c->serial_chain, c->rxs, c->rxs_ld, c->rx_part, c->row_grid, c->force_exact);
@@ -1274,6 +1297,7 @@ static inline void launch_rest(fnn_ctx* c) {
     k_chain<<<1, PICK_THREADS, c->chain_smem, cs>>>(c->Sx, c->st, c->stage, c->serial_chain, c->chain_stage_cap);
     k_patch<<<PATCH_BLOCKS, PATCH_THREADS, 0, cs>>>(c->D, c->ld, c->Sx, c->pos, c->st, c->patch_part);
     if (c->overlap) { cudaEventRecord(c->ev_join, c->stream2); c->join_pending = true; }
+    return FNN_OK;
 }
 // the forked branch has to be back on the main stream before a capture ends, before the state is read, before the next run
 static inline void join_branch(fnn_ctx* c) {
@@ -1331,6 +1355,8 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
                                                           c->tl, c->tl_iter0, c->tl_count);
     k_rowsum<<<(ni + 127) / 128, 128, 0, c->stream>>>(c->D, c->ld, ni, c->Sx, c->st);
     FNN_CUDA(cudaGetLastError());
+    // iterations in which no strategy runs keep a zero record row; the strategy kernels fill the others
+    if (c->record) FNN_CUDA(cudaMemsetAsync(c->record, 0, sizeof(long long) * rec::COLS * (n + 8), c->stream));
     int64_t launches = 2, scans = 0;
     const int64_t max_iters = n;  // n-3 .. n-1 iterations; kernels no-op once done
     double prof_ms = 0.0, prof_bytes = 0.0;
@@ -1363,7 +1389,7 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
                 if (c->h_st->done) break;
                 FNN_CUDA(cudaEventRecord(p0, c->stream));
             }
-            launch_scan(c);
+            if (int rc = launch_scan(c)) return rc;
             if (sample) {
                 FNN_CUDA(cudaEventRecord(p1, c->stream));
                 FNN_CUDA(cudaEventSynchronize(p1));
@@ -1374,7 +1400,7 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
                 prof_bytes += 4.0 * mm * (mm - 1.0) - 8.0 * pp + 8.0 * mm;
                 ++prof_samples;
             }
-            launch_rest(c);
+            if (int rc = launch_rest(c)) return rc;
             launches += c->launches_per_iter(); ++scans;
         }
         join_branch(c);
@@ -1383,18 +1409,21 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
         constexpr int GI = 32;  // iterations per graph
         if (!c->graph) {
             cudaGraph_t g;
+            int rc = FNN_OK;
             FNN_CUDA(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-            for (int i = 0; i < GI; ++i) { launch_scan(c); launch_rest(c); }
+            for (int i = 0; i < GI && !rc; ++i) { rc = launch_scan(c); if (!rc) rc = launch_rest(c); }
             join_branch(c);
             FNN_CUDA(cudaStreamEndCapture(c->stream, &g));
+            if (rc) { cudaGraphDestroy(g); return rc; }
             FNN_CUDA(cudaGraphInstantiate(&c->graph, g, 0));
             cudaGraphDestroy(g);
             c->graph_iters = GI;
             if (c->o.mode != FNN_CANONICAL) {
                 FNN_CUDA(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-                for (int i = 0; i < GI; ++i) launch_rest(c);
+                for (int i = 0; i < GI && !rc; ++i) rc = launch_rest(c);
                 join_branch(c);
                 FNN_CUDA(cudaStreamEndCapture(c->stream, &g));
+                if (rc) { cudaGraphDestroy(g); return rc; }
                 FNN_CUDA(cudaGraphInstantiate(&c->graph_strategy, g, 0));
                 cudaGraphDestroy(g);
             }
@@ -1420,7 +1449,8 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
         int64_t it = 0;
         while (it < max_iters) {
             for (int b = 0; b < 256 && it < max_iters; ++b, ++it) {
-                launch_scan(c); launch_rest(c);
+                if (int rc = launch_scan(c)) return rc;
+                if (int rc = launch_rest(c)) return rc;
                 launches += c->launches_per_iter(); ++scans;
             }
             join_branch(c);
@@ -1492,6 +1522,17 @@ extern "C" int64_t fnn_ctx_trace(fnn_ctx* c, double* rows, int64_t max_rows) {
     int64_t k = std::min<int64_t>(c->trace_rows, max_rows);
     if (cudaMemcpy(rows, c->trace, sizeof(double) * 8 * k, cudaMemcpyDeviceToHost) != cudaSuccess) {
         fnn::set_error("trace copy failed: %s", cudaGetErrorString(cudaGetLastError()));
+        return FNN_E_CUDA;
+    }
+    return k;
+}
+
+extern "C" int64_t fnn_ctx_strategy_record(fnn_ctx* c, int64_t* rows, int64_t max_rows) {
+    if (!c || !rows || !c->record) { fnn::set_error("fnn_ctx_strategy_record: record not kept (opts.record_trace)"); return FNN_E_STATE; }
+    cudaSetDevice(c->o.device);
+    int64_t k = std::min<int64_t>(c->trace_rows, max_rows);
+    if (cudaMemcpy(rows, c->record, sizeof(long long) * rec::COLS * k, cudaMemcpyDeviceToHost) != cudaSuccess) {
+        fnn::set_error("strategy record copy failed: %s", cudaGetErrorString(cudaGetLastError()));
         return FNN_E_CUDA;
     }
     return k;

@@ -51,7 +51,8 @@ enum fnn_mode {
  * hard-coded constants it buries (SURVEY.md §5 "config / flags"). */
 typedef struct fnn_opts {
     int32_t mode;               /* -mode, enum fnn_mode; default canonical */
-    int32_t mult;               /* -mult, default 5 (NeighborNetRandom.java:47) */
+    int32_t mult;               /* -mult, default 5 (NeighborNetRandom.java:47); the Random modes need mult >= 1 (with no draw
+                                   the reference has no pair to join), fnn_ctx_create returns FNN_E_ARG otherwise */
     int32_t additive;           /* -additive (NeighborNetLocal.java:223) */
     int32_t canonical_fallback; /* 1024: num_active <= this uses the canonical scan (NetMakerOriginal.java:361) */
     int64_t seed;               /* java.util.Random(seed) stream for Relaxed/Random (reference is unseedable) */
@@ -111,6 +112,15 @@ int fnn_ctx_read_matrix(fnn_ctx* c, double* D_rowmajor_out);
 int fnn_ctx_order(fnn_ctx* c, int32_t* ordering_out);
 /* per-iteration trace rows of 8 doubles (m, c, Cx.id, Cy.id, x.id, y.id, kind, best); returns rows written */
 int64_t fnn_ctx_trace(fnn_ctx* c, double* rows_out, int64_t max_rows);
+/* per-iteration strategy record, kept with the trace (opts.record_trace = 1; otherwise FNN_E_STATE): rows of 4 int64, one
+ * per trace row; returns rows written.  A row is what the selection strategy did in that iteration's findNodes:
+ *   Random:  draws, draws whose nextInt rejected at least once, draws remapped because j hit i or i.nbr
+ *            (NeighborNetRandom.java:144-157), digest of the drawn (i, j) positions;
+ *   Relaxed: row scans, tie entries they returned, -additive look-aheads, digest of the scanned rows and their ties;
+ *   all zero where the strategy did not run (canonical mode, m <= canonical_fallback, the last iteration).
+ * The digest (a uint64 stored as int64) is defined in csrc/fnn_record.h; a test hook for holding the strategies to a CPU
+ * restatement draw for draw. */
+int64_t fnn_ctx_strategy_record(fnn_ctx* c, int64_t* rows_out, int64_t max_rows);
 int fnn_ctx_stats(fnn_ctx* c, fnn_stats* out);
 /* device pointer + leading dimension of the internal matrix (for zero-copy producers such as torch) */
 int fnn_ctx_matrix_ptr(fnn_ctx* c, double** dptr, int64_t* ld);

@@ -12,6 +12,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
+_RELAXED_SM = False
 
 MODES = {"canonical": 0, "relaxed": 1, "random_n": 2, "random_nlogn": 3, "random_logn": 4}
 
@@ -27,6 +28,7 @@ def lib():
         srcs = [os.path.join(_HERE, f) for f in ("nnet_oracle.cpp", "csw_l1.cpp")]
         srcs.append(os.path.join(os.path.dirname(_HERE), "fastneighbornet_b200", "csrc", "fnn_relaxed_sm.h"))
         srcs.append(os.path.join(os.path.dirname(_HERE), "fastneighbornet_b200", "csrc", "fnn_tile_iter.h"))
+        srcs.append(os.path.join(os.path.dirname(_HERE), "fastneighbornet_b200", "csrc", "fnn_record.h"))
         if not os.path.exists(so) or any(os.path.exists(s_) and os.path.getmtime(s_) > os.path.getmtime(so) for s_ in srcs):
             build()
         L = ctypes.CDLL(so)
@@ -35,7 +37,7 @@ def lib():
         c_lp = ctypes.POINTER(ctypes.c_int64)
         L.oracle_order.argtypes = [ctypes.c_int, ctypes.c_int64, c_dp, ctypes.c_int64, ctypes.c_int, ctypes.c_int,
                                    ctypes.c_int, c_ip, c_dp, ctypes.c_int64, c_lp, c_lp, ctypes.c_int, c_dp,
-                                   ctypes.c_int64]
+                                   ctypes.c_int64, c_lp]
         L.oracle_order.restype = ctypes.c_int
         L.oracle_rowsums.argtypes = [ctypes.c_int64, c_dp, c_dp]
         L.oracle_setup_d.argtypes = [ctypes.c_int64, c_ip, c_dp, c_dp]
@@ -73,11 +75,16 @@ def _bp(a):
     return a.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8))
 
 
-def order(D, mode="canonical", seed=12345, mult=5, additive=False, fallback=1024, want_trace=True, threads=1, max_iters=0):
+def order(D, mode="canonical", seed=12345, mult=5, additive=False, fallback=1024, want_trace=True, threads=1, max_iters=0,
+          want_record=False):
     """Returns (ordering[n+1] int32, trace[k,8] float64, counters dict).  D is copied.
     max_iters = K > 0: stop after K agglomeration iterations; the trace is then the first K rows of the full trace and the
-    ordering is undefined (all zeros).  0 = no limit."""
+    ordering is undefined (all zeros).  0 = no limit.
+    want_record: counters["record"] is the strategy record of fnn_ctx_strategy_record, one row per trace row ([k,4] int64,
+    digest in column 3; view it as uint64).  Relaxed then runs through the product's state machine (set_relaxed_sm), which
+    asks for the row scans in the device's order; tests/test_relaxed_sm_cpu.py holds it to the literal restatement."""
     n = D.shape[0]
+    want_trace = want_trace or want_record
     Dc = np.array(D, dtype=np.float64, order="C", copy=True)
     ordering = np.zeros(n + 1, dtype=np.int32)
     max_trace = n + 8
@@ -85,12 +92,22 @@ def order(D, mode="canonical", seed=12345, mult=5, additive=False, fallback=1024
     ntr = np.zeros(1, dtype=np.int64)
     cnt = np.zeros(2, dtype=np.int64)
     ab = np.zeros(1, dtype=np.float64)
-    rc = lib().oracle_order(MODES[mode], n, _dp(Dc), seed, mult, int(additive), fallback, _ip(ordering),
-                            _dp(trace) if want_trace else None, max_trace, _lp(ntr), _lp(cnt), int(threads), _dp(ab), int(max_iters))
+    record = np.zeros((max_trace, 4), dtype=np.int64)
+    sm_before = _RELAXED_SM
+    if want_record and mode == "relaxed":
+        set_relaxed_sm(True)
+    try:
+        rc = lib().oracle_order(MODES[mode], n, _dp(Dc), seed, mult, int(additive), fallback, _ip(ordering),
+                                _dp(trace) if want_trace else None, max_trace, _lp(ntr), _lp(cnt), int(threads), _dp(ab),
+                                int(max_iters), _lp(record) if want_record else None)
+    finally:
+        set_relaxed_sm(sm_before)
     if rc != 0:
         raise RuntimeError(f"oracle_order rc={rc}")
-    return ordering, trace[: int(ntr[0])], {"pair_evals": int(cnt[0]), "npe_would_fire": int(cnt[1]), "D_final": Dc,
-                                             "alg_bytes": float(ab[0])}
+    out = {"pair_evals": int(cnt[0]), "npe_would_fire": int(cnt[1]), "D_final": Dc, "alg_bytes": float(ab[0])}
+    if want_record:
+        out["record"] = record[: int(ntr[0])]
+    return ordering, trace[: int(ntr[0])], out
 
 
 def rowsums(D):
@@ -189,4 +206,6 @@ def l1_split_weights(n, d_pos, max_cg_iters=0, max_cg_calls=0, with_active=False
 def set_relaxed_sm(on):
     """Route the oracle's Relaxed findNodes through the PRODUCT's control state machine (csrc/fnn_relaxed_sm.h), with the
     oracle's own row scans: used by tests to hold that state machine against the literal restatement on the CPU."""
+    global _RELAXED_SM
     lib().oracle_set_relaxed_sm(int(bool(on)))
+    _RELAXED_SM = bool(on)

@@ -37,6 +37,8 @@
 // held against the literal findNodes below (tests/test_relaxed_sm_cpu.py); the oracle never depends on it otherwise
 #include "../fastneighbornet_b200/csrc/fnn_relaxed_sm.h"
 #include "../fastneighbornet_b200/csrc/fnn_tile_iter.h"
+// the digest of the product's per-iteration strategy record (fnn_ctx_strategy_record)
+#include "../fastneighbornet_b200/csrc/fnn_record.h"
 
 namespace {
 static int g_use_relaxed_sm = 0;
@@ -160,6 +162,8 @@ struct Engine {
     int threads = 1;             // >1: NeighborNetCanonical's thread-pool partition (NeighborNetCanonical.java:180-206)
     std::unique_ptr<SlicePool> pool;
     std::vector<TraceRow>* trace = nullptr;
+    std::vector<int64_t>* record = nullptr;   // rec::COLS per iteration, as fnn_ctx_strategy_record returns it
+    int64_t* rec_row = nullptr;               // this iteration's row (null: no record kept)
     int status = 0;
     int64_t max_iters = 0;       // >0: stop after this many agglomeration iterations (the ordering is then undefined)
     bool stopped = false;
@@ -533,6 +537,7 @@ struct Engine {
         SMView nv{this, num_active};
         relaxed::begin_call(SM, (int)n);
         int look_accept = 0;
+        int nscan = 0;
         while (true) {
             const relaxed::Request rq = relaxed::step(SM, nv, look_accept);
             if (rq == relaxed::REQ_DONE) break;
@@ -551,8 +556,16 @@ struct Engine {
                     if (Qpq < myMin) { myMin = Qpq; cnt = 0; if (cnt < room) out[cnt] = row; cnt = 1; }
                     else if (Qpq == myMin) { if (cnt < room) out[cnt] = row; ++cnt; }
                 }
+                if (rec_row) {   // scans, ties, digest of fnn_record.h
+                    uint64_t dg = rec::scan_term(nscan, SM.req_pos, -1, 0);
+                    for (int r = 0; r < cnt && r < room; ++r) dg += rec::scan_term(nscan, SM.req_pos, r, out[r]);
+                    rec_row[0] += 1; rec_row[1] += cnt;
+                    rec_row[3] = (int64_t)((uint64_t)rec_row[3] + dg);
+                }
+                ++nscan;
                 if (cnt > room || !relaxed::commit_scan(SM, cnt)) { status = -12; break; }
             } else {   // REQ_LOOKAHEAD
+                if (rec_row) rec_row[2] += 1;
                 const int cx = act[SM.cx_pos], cy = act[SM.cy_pos], t = act[SM.look_test_pos];
                 const double originalQ = ((double)num_clusters - 2.0) * clusterDist(cx, t) - nd[cx].Sx - nd[t].Sx;
                 const double newQ = findAgglomeratedQ(cx, cy, t, num_clusters, num_active);
@@ -580,17 +593,25 @@ struct Engine {
         int i = rng.nextInt(num_active);
         int j;
         Cx = Cy = -1;
+        if (rec_row) rec_row[0] = searchAmount;
         for (int64_t k = 0; k < searchAmount; ++k) {
+            const uint64_t one_step = (rng.s * 0x5DEECE66DULL + 0xBULL) & ((1ULL << 48) - 1);
+            int j0;
             if (nd[act[i]].nbr >= 0) {
                 int iNbr = nd[nd[act[i]].nbr].pos;
-                j = rng.nextInt(num_active - 2);
+                j = j0 = rng.nextInt(num_active - 2);
                 if (i == j && num_active - 1 == iNbr) j = num_active - 2;
                 else if (i == j && num_active - 1 != iNbr) j = num_active - 1;
                 else if (iNbr == j && num_active - 2 == i) j = num_active - 1;
                 else if (iNbr == j && num_active - 2 != i) j = num_active - 2;
             } else {
-                j = rng.nextInt(num_active - 1);
+                j = j0 = rng.nextInt(num_active - 1);
                 if (i == j) j = num_active - 1;
+            }
+            if (rec_row) {   // nextInt rejected (took more than one LCG step); remapped; digest of fnn_record.h
+                rec_row[1] += rng.s != one_step;
+                rec_row[2] += j != j0;
+                rec_row[3] = (int64_t)((uint64_t)rec_row[3] + rec::draw_term(k, i, j));
             }
             int p = act[i], q = act[j];
             double Dpq = clusterDist(p, q);
@@ -701,6 +722,10 @@ struct Engine {
         int num_active = num_nodes, num_clusters = num_nodes;
         for (int64_t iter = 0; num_active > 3; ++iter) {
             if (max_iters > 0 && iter >= max_iters) { stopped = true; break; }
+            if (record) {   // a zero row unless the strategy runs in this iteration
+                record->insert(record->end(), rec::COLS, 0);
+                rec_row = record->data() + record->size() - rec::COLS;
+            }
             if (num_active == 4 && num_clusters == 2) {
                 int p = act[0];
                 int q = (nd[p].nbr != act[1]) ? act[1] : act[2];
@@ -978,12 +1003,14 @@ void oracle_set_relaxed_sm(int on) { g_use_relaxed_sm = on; }
 
 // Ordering.  D is n*n row-major and is mutated in place (like the Java double[][]).
 // trace_out: optional [max_trace][8] doubles (m,c,cx,cy,x,y,kind,best); returns rows in *n_trace.
+// record_out: optional [max_trace][4] int64, the strategy record of fnn_ctx_strategy_record (Relaxed: only through the
+// product's state machine, oracle_set_relaxed_sm(1), whose scan sequence is the device's); requires trace_out.
 // max_iters > 0: stop after that many agglomeration iterations and return the trace so far (a prefix of the full trace);
 // the ordering is then all zeros.  0 = run to the end.
 int oracle_order(int mode, int64_t n, double* D, int64_t seed, int mult, int additive, int fallback,
                  int32_t* ordering, double* trace_out, int64_t max_trace, int64_t* n_trace,
                  int64_t* counters /* [0]=pair_evals [1]=npe_would_fire */, int threads, double* alg_bytes,
-                 int64_t max_iters) {
+                 int64_t max_iters, int64_t* record_out) {
     Engine e;
     e.n = n; e.D = D; e.mode = mode; e.mult = mult; e.additive = additive != 0; e.fallback = fallback;
     e.max_iters = max_iters;
@@ -991,7 +1018,13 @@ int oracle_order(int mode, int64_t n, double* D, int64_t seed, int mult, int add
     e.threads = threads < 1 ? 1 : threads;
     std::vector<TraceRow> tr;
     if (trace_out) e.trace = &tr;
+    std::vector<int64_t> rc_rows;
+    if (record_out) e.record = &rc_rows;
     int rc = e.run(ordering);
+    if (record_out) {   // one row per trace row (the record is only kept together with the trace)
+        const int64_t k = std::min<int64_t>((int64_t)rc_rows.size() / rec::COLS, max_trace);
+        std::copy(rc_rows.begin(), rc_rows.begin() + rec::COLS * k, record_out);
+    }
     if (trace_out) {
         int64_t k = std::min<int64_t>((int64_t)tr.size(), max_trace);
         for (int64_t i = 0; i < k; ++i) {

@@ -10,6 +10,20 @@ Citations are file:line into /root/reference.
 import math
 
 DBL_MAX = 1.7976931348623157e308
+M64 = (1 << 64) - 1
+
+
+def splitmix64(z):
+    """splitmix64's output function (Steele, Lea, Flood 2014), mod 2**64: restated here independently of csrc/fnn_record.h."""
+    z = (z + 0x9E3779B97F4A7C15) & M64
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & M64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & M64
+    return z ^ (z >> 31)
+
+
+def draw_digest_term(k, i, j):
+    """The strategy record's term for draw k of an iteration going from position i to position j."""
+    return splitmix64(splitmix64(k) ^ (((i & 0xFFFFFFFF) << 32) | (j & 0xFFFFFFFF)))
 
 
 class JavaRandom:
@@ -17,8 +31,10 @@ class JavaRandom:
 
     def __init__(self, seed):
         self.s = (seed ^ 0x5DEECE66D) & ((1 << 48) - 1)
+        self.calls = 0  # LCG steps taken
 
     def _next(self, bits):
+        self.calls += 1
         self.s = (self.s * 0x5DEECE66D + 0xB) & ((1 << 48) - 1)
         v = self.s >> (48 - bits)
         if v >= 1 << 31:
@@ -70,6 +86,7 @@ class NeighborNet:
         self.first_time = True
         self.top = 0
         self.row_perm = []
+        self.record = []  # Random modes: per iteration [draws, rejected, remapped, digest] (fnn_ctx_strategy_record)
 
     # the cluster-distance ladder, e.g. NetMakerOriginal.java:218-225
     def dpq(self, p, q):
@@ -192,10 +209,13 @@ class NeighborNet:
         amount = {"random_logn": lg, "random_n": num_active, "random_nlogn": lg * num_active}[self.mode] * self.mult
         i = self.rng.next_int(num_active)
         self.Cx = self.Cy = None
-        for _ in range(amount):
+        row = self.record[-1]
+        row[0] = amount
+        for k in range(amount):
+            calls_before = self.rng.calls
             if nodes[i].nbr is not None:
                 inbr = nodes[i].nbr.positionID
-                j = self.rng.next_int(num_active - 2)
+                j = j0 = self.rng.next_int(num_active - 2)
                 if i == j and num_active - 1 == inbr:
                     j = num_active - 2
                 elif i == j and num_active - 1 != inbr:
@@ -205,9 +225,12 @@ class NeighborNet:
                 elif inbr == j and num_active - 2 != i:
                     j = num_active - 2
             else:
-                j = self.rng.next_int(num_active - 1)
+                j = j0 = self.rng.next_int(num_active - 1)
                 if i == j:
                     j = num_active - 1
+            row[1] += self.rng.calls - calls_before > 1
+            row[2] += j != j0
+            row[3] = (row[3] + draw_digest_term(k, i, j)) & M64
             p, q = nodes[i], nodes[j]
             Q = (float(num_clusters) - 2.0) * self.dpq(p, q) - p.Sx - q.Sx
             if (self.Cx is None or Q < self.best) and p.nbr is not q:
@@ -334,6 +357,7 @@ class NeighborNet:
         D, nodes = self.D, self.nodes
         num_active = num_clusters = num_nodes
         while num_active > 3:
+            self.record.append([0, 0, 0, 0])
             if num_active == 4 and num_clusters == 2:
                 p = nodes[0]
                 q = nodes[1] if p.nbr is not nodes[1] else nodes[2]
