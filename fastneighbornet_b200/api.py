@@ -62,6 +62,7 @@ ABI_SYMBOLS = [
     "fnn_split_weights", "fnn_csw_matvec", "fnn_ctx_ipc_handle", "fnn_ctx_connect", "fnn_weighted_splits", "fnn_network",
     "fnn_phylip_taxa", "fnn_read_phylip", "fnn_write_nexus", "fnn_java_double_to_string", "fnn_release_cache",
     "fnn_ctx_load_host_rows", "fnn_ctx_commit_load", "fnn_split_weights_budget", "fnn_ctx_strategy_record",
+    "fnn_ctx_prune_bounds",
 ]
 
 
@@ -96,6 +97,9 @@ def lib():
         L.fnn_ctx_trace.argtypes = [vp, c_dp, ctypes.c_int64]
         L.fnn_ctx_trace.restype = ctypes.c_int64
         L.fnn_ctx_strategy_record.argtypes = [vp, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64]
+        L.fnn_ctx_prune_bounds.argtypes = [vp, ctypes.c_int64, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double),
+                                           ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_double),
+                                           ctypes.POINTER(ctypes.c_int64)]
         L.fnn_ctx_strategy_record.restype = ctypes.c_int64
         L.fnn_ctx_stats.argtypes = [vp, ctypes.POINTER(fnn_stats)]
         L.fnn_ctx_matrix_ptr.argtypes = [vp, ctypes.POINTER(vp), ctypes.POINTER(ctypes.c_int64)]
@@ -138,7 +142,7 @@ def device_count():
 
 
 # A/B switches carried in fnn_opts.reserved (include/fastnn.h): name -> (index, bit or None for "whole int")
-_RESERVED = {"serial_chain": (1, None), "no_overlap": (5, 1), "force_exact_pick": (5, 2), "csw_variant": (4, None)}
+_RESERVED = {"no_prune": (0, None), "serial_chain": (1, None), "no_overlap": (5, 1), "force_exact_pick": (5, 2), "csw_variant": (4, None)}
 CSW_VARIANTS = {"default": 0, "graph": 1, "literal": 2}
 
 
@@ -296,6 +300,25 @@ class Context:
             _check(int(k))
         return rows[: int(k)]
 
+    def prune_bounds(self, iters):
+        """State of the scan's pruning bounds after the first `iters` iterations (fnn_ctx_prune_bounds; consumes the loaded
+        matrix): dict with D (slot layout), segmin (n, S), smax (S,) decoded to float64 (NaN = none), Sx, m, P2, mask_su,
+        iter, done."""
+        n = self.n
+        S = (((n + 15) // 16 * 16) + 255) // 256
+        D = np.empty((n, n)); segmin = np.empty((n, S)); sx = np.empty(n)
+        keys = np.zeros(S, dtype=np.uint64); meta = np.zeros(6, dtype=np.int64)
+        _check(lib().fnn_ctx_prune_bounds(self._h, int(iters), _dp(D), _dp(segmin),
+                                          keys.ctypes.data_as(ctypes.POINTER(ctypes.c_uint64)), _dp(sx),
+                                          meta.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))))
+        assert int(meta[4]) == S
+        top = (keys >> np.uint64(63)).astype(bool)
+        bits = np.where(top, keys & np.uint64(0x7FFFFFFFFFFFFFFF), ~keys)
+        smax = bits.view(np.float64).copy()
+        smax[keys == 0] = np.nan
+        return {"D": D, "segmin": segmin, "smax": smax, "Sx": sx, "m": int(meta[0]), "P2": int(meta[1]),
+                "mask_su": int(meta[2]), "iter": int(meta[3]), "done": int(meta[5])}
+
     def stats(self):
         s = fnn_stats()
         _check(lib().fnn_ctx_stats(self._h, ctypes.byref(s)))
@@ -304,6 +327,8 @@ class Context:
         out["picks_exact"] = int(s.reserved[1])       # ... that needed the exact left-to-right sums
         out["strategy_alg_bytes"] = float(s.reserved[2])   # Relaxed row scans / Random samples (SURVEY 8d K7/K9)
         out["strategy_units"] = int(s.reserved[3])
+        out["scan_read_bytes"] = float(s.reserved[4])      # matrix bytes the selection scan fetched (pruned segments not)
+        out["scan_units_skipped"] = int(s.reserved[5])     # row segments the pruned scans did not fetch
         return out
 
 

@@ -99,6 +99,10 @@ struct DevState {
     // iterations, the only way to see the real overlap and gaps inside a graph replay
     unsigned long long* tl;
     int tl_iter0, tl_count;
+    // ---- pruning of the selection scan (k_prune): whether this launch reads only the surviving row segments, and counters
+    int prune_on, pad2;
+    unsigned long long read_bytes;      // matrix bytes the scan fetched (pruned launches: surviving segments; others: algorithmic)
+    unsigned long long units_skipped;   // row segments (a pair row counts once) the pruned launches did not fetch
 };
 constexpr int TL_EVENTS = 16;
 enum { TL_SCAN0 = 0, TL_SCAN1, TL_RX0, TL_RX1, TL_PICK0, TL_PICK1, TL_ROWS0, TL_ROWS1, TL_SCAT0, TL_SCAT1, TL_CHAIN0, TL_CHAIN1,
@@ -182,19 +186,35 @@ __global__ void k_init_nodes(int n, int* id, int* pos, int* p2s, DevState* st, i
     }
 }
 
+// Pruning bounds of the selection scan (k_prune).  segmin[r * sld + b] is a lower bound on every entry D[r][c] with c a live
+// slot in the 256-column segment b, c != r and c not r's pair partner; smax[b] is the largest Sx of the representatives of
+// segment b except the masked new cluster, as an order-preserving key (0 = unknown: decodes to NaN, which prunes nothing).
+constexpr int SEG = 256;
+__device__ __forceinline__ unsigned long long ord_key(double x) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double ord_val(unsigned long long k) {
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
+}
+
 // K1: Sx[k] = sum_{j != k} D[k][j], ascending j (NetMakerOriginal.java:164-191).  Thread k walks
-// column k (== row k by symmetry) so that a warp reads 256 contiguous bytes per step.
-__global__ void k_rowsum(const double* __restrict__ D, int64_t ld, int n, double* Sx, DevState* st) {
+// column k (== row k by symmetry) so that a warp reads 256 contiguous bytes per step; on the way it records the
+// segment minima of row k and the segment maxima of Sx.
+__global__ void k_rowsum(const double* __restrict__ D, int64_t ld, int n, double* Sx, DevState* st, double* segmin, int64_t sld,
+                         unsigned long long* smax) {
     int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
-    double s = 0.0, mx = 0.0;
+    double s = 0.0, mx = 0.0, mn = INFINITY;
     const double* col = D + k;
 #pragma unroll 8
     for (int j = 0; j < n; ++j) {
         double v = col[(int64_t)j * ld];
-        if (j != k) { s += v; mx = fmax(mx, fabs(v)); }
+        if (j != k) { s += v; mx = fmax(mx, fabs(v)); mn = v < mn ? v : mn; }
+        if (segmin && ((j + 1) % SEG == 0 || j + 1 == n)) { segmin[(int64_t)k * sld + j / SEG] = mn; mn = INFINITY; }
     }
     Sx[k] = s;
+    if (smax) atomicMax(&smax[k / SEG], ord_key(s));
     // non-negative doubles order like their bit patterns
     if (st) atomicMax(reinterpret_cast<unsigned long long*>(&st->Dmax), (unsigned long long)__double_as_longlong(mx));
 }
@@ -337,7 +357,9 @@ k_rx_stage(const double* __restrict__ D, int64_t ld, const int* __restrict__ id,
             st->cx = sel.cx; st->cxn = sel.cxn; st->cy = sel.cy; st->cyn = sel.cyn; st->need_rx = sel.need_rx;
             if (!strategy && sel.cx >= 0) {
                 st->selQ = sel.q; st->sel_i = sel.i; st->sel_j = sel.j;
-                st->alg_bytes += 4.0 * (double)m_ * ((double)m_ - 1.0) - 4.0 * (double)st->P2 + 8.0 * (double)m_;
+                const double ab = 4.0 * (double)m_ * ((double)m_ - 1.0) - 4.0 * (double)st->P2 + 8.0 * (double)m_;
+                st->alg_bytes += ab;
+                if (!st->prune_on) st->read_bytes += (unsigned long long)ab;
             }
             tl_stamp(st, TL_RX0);
         }
@@ -667,7 +689,7 @@ __device__ __forceinline__ double sub_dist(const double* D, int64_t ld, int p, b
 
 // ------------------------------------------------------------------ K4+K5a: subtract sweep + build changed rows
 __global__ void __launch_bounds__(256)
-k_rows(const double* __restrict__ D, int64_t ld, double* Sx, DevState* st, double* scratch) {
+k_rows(const double* __restrict__ D, int64_t ld, double* Sx, DevState* st, double* scratch, unsigned long long* smax) {
     if (st->done || st->skip) return;
     if (blockIdx.x == 0 && threadIdx.x == 0) tl_stamp(st, TL_ROWS0);
     const int m = st->m, P2 = st->P2, m_new = st->m_new, K = st->K;
@@ -680,6 +702,7 @@ k_rows(const double* __restrict__ D, int64_t ld, double* Sx, DevState* st, doubl
     const double Duv = st->Duv;
 
     for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < m; t += gridDim.x * blockDim.x) {
+        if (t * SEG < m) smax[t] = 0ull;   // k_scatter rebuilds the segment maxima of Sx from the final values
         // ---- role 1: subtract old cluster distances (old layout), bystander representatives only
         {
             const int s = t;
@@ -727,7 +750,8 @@ k_rows(const double* __restrict__ D, int64_t ld, double* Sx, DevState* st, doubl
 // its u.Sx is summed by k_chain + k_patch concurrently with that scan.
 __global__ void __launch_bounds__(256)
 k_scatter(double* D, int64_t ld, double* Sx, const int* __restrict__ pos, DevState* st, const double* __restrict__ scratch,
-          double* stage, const int* __restrict__ id, const int* __restrict__ p2s) {
+          double* stage, const int* __restrict__ id, const int* __restrict__ p2s, double* segmin, int64_t sld,
+          unsigned long long* smax) {
     if (st->done || st->skip) return;
     __shared__ bool amLast;
     if (blockIdx.x == 0 && threadIdx.x == 0) tl_stamp(st, TL_SCAT0);
@@ -740,20 +764,27 @@ k_scatter(double* D, int64_t ld, double* Sx, const int* __restrict__ pos, DevSta
     __syncthreads();
     const double* r0 = scratch;        // row of u  (chg index 0 is always su)
     const double* r1 = scratch + ld;   // row of u' (chg index 1 is always su+1)
-    for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < m_new; t += gridDim.x * blockDim.x) {
+    // one slot t: returns the ord_key of its final Sx if t is an unmasked representative, else 0
+    auto slot = [&](int t) -> unsigned long long {
+        bool changed = false;
+        for (int k = 0; k < K; ++k) changed |= (cslot[k] == t);
         for (int k = 0; k < K; ++k) {
             const double v = scratch[(int64_t)k * ld + t];
             const int s = cslot[k];
             D[(int64_t)s * ld + t] = v;
             D[(int64_t)t * ld + s] = v;
+            if (!changed) {   // the changed rows themselves are recomputed below
+                double* sm = segmin + (int64_t)t * sld + s / SEG;
+                if (v < *sm) *sm = v;
+            }
         }
         // add new cluster distances (updateClusterDistances, :517-536)
         const bool pPair = t < P2n;
-        if (pPair && (t & 1)) continue;
+        if (pPair && (t & 1)) return 0ull;
         if (t == su) {
             stage[sidx(pos[t])] = 0.0;
             stage[sidx(pos[t + 1])] = 0.0;
-            continue;
+            return 0ull;
         }
         double base0 = Sx[t], base1 = pPair ? Sx[t + 1] : 0.0;
         for (int k = 0; k < K; ++k) {
@@ -763,9 +794,43 @@ k_scatter(double* D, int64_t ld, double* Sx, const int* __restrict__ pos, DevSta
         double dpu;
         if (pPair) dpu = (((r0[t] + r1[t]) + r0[t + 1]) + r1[t + 1]) * 0.25;
         else dpu = (r0[t] + r1[t]) * 0.5;
-        Sx[t] = base0 + dpu;
+        const double sx = base0 + dpu;
+        Sx[t] = sx;
         stage[sidx(pos[t])] = dpu;
         if (pPair) { Sx[t + 1] = base1 + dpu; stage[sidx(pos[t + 1])] = 0.0; }
+        return ord_key(sx);
+    };
+    // blockDim.x divides SEG: the threads of a warp share one segment, so one atomic per warp
+    for (int t0 = blockIdx.x * blockDim.x; t0 < m_new; t0 += gridDim.x * blockDim.x) {
+        const int t = t0 + threadIdx.x;
+        unsigned long long key = t < m_new ? slot(t) : 0ull;
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            const unsigned long long o = __shfl_xor_sync(0xffffffffu, key, off);
+            key = o > key ? o : key;
+        }
+        if ((threadIdx.x & 31) == 0 && key) atomicMax(&smax[t / SEG], key);
+    }
+    // segment minima of the changed rows, from their new contents (one warp per row segment)
+    {
+        const int nseg = (m_new + SEG - 1) / SEG, lane = threadIdx.x & 31;
+        for (int u = (blockIdx.x * blockDim.x + threadIdx.x) / 32; u < K * nseg; u += gridDim.x * blockDim.x / 32) {
+            const int k = u / nseg, b = u % nseg, s = cslot[k], partner = s < P2n ? (s ^ 1) : -1;
+            double mn = INFINITY;
+            for (int i = lane; i < SEG; i += 32) {
+                const int col = b * SEG + i;
+                if (col < m_new && col != s && col != partner) {
+                    const double v = scratch[(int64_t)k * ld + col];
+                    mn = v < mn ? v : mn;
+                }
+            }
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) {
+                const double o = __shfl_xor_sync(0xffffffffu, mn, off);
+                mn = o < mn ? o : mn;
+            }
+            if (lane == 0) segmin[(int64_t)s * sld + b] = mn;
+        }
     }
     // ---- commit: every block has read the event descriptor before it arrives here
     __threadfence();
@@ -918,6 +983,113 @@ k_patch(const double* __restrict__ D, int64_t ld, const double* __restrict__ Sx,
     }
 }
 
+// ------------------------------------------------------------------ K2a: which row segments the selection scan must read
+// Every pair of row cluster r and a column cluster of 256-column segment b has Q >= LB(r, b) = (c-2)*segmin(r, b) - Sx(r) -
+// smax(b): a 2- or 4-entry pair mean is never below the smallest entry.  T is the exactly evaluated Q of a real, unmasked pair
+// (the previous launch's per-CTA winners re-evaluated with the current Sx and c, so T >= the minimum the scan looks for).  A
+// unit - one single row, or one pair row (p, p+1), across one segment - is skipped only when LB > T + eps, strictly: it then
+// cannot hold a pair with Q <= T, so the minimum, its ties and the (Q, i, j) min-loc are unchanged.
+// eps = 2*delta, delta the filter slack of k_scan_tma: the exact Q of a pair is within delta of its real value (the filter's
+// derivation bounds each of its two forms by that much), LB's three roundings of values of the same magnitude bound
+// ((c-2)*max|D| + 2c*max|D|) plus one 2^-1075 on underflow stay within another delta, and so does the rounding of T + eps.
+constexpr int PRUNE_MIN_M = 4096;   // below this the scan is short and k_prune's launch would cost more than it saves
+constexpr int PRUNE_THREADS = 256;
+
+// the reference's exact, role-ordered Q of the pair named by a min-loc key, in the scan's operand order (fnn_scan_tma.cuh
+// exact1 / exact_pp); +inf if the key does not name two live, unmasked clusters of the current layout
+__device__ double seed_q(const double* __restrict__ D, int64_t ld, const double* __restrict__ Sx, const int* __restrict__ p2s,
+                         int m, int P2, int msk, double cm2, unsigned long long key) {
+    const unsigned i = (unsigned)(key >> 32), j = (unsigned)(key & 0xffffffffu);
+    if (i >= (unsigned)m || j >= (unsigned)m || i == j) return INFINITY;
+    const int si = p2s[i], sj = p2s[j];
+    if (si < 0 || si >= m || sj < 0 || sj >= m || si == sj) return INFINITY;
+    if ((si < P2 && (si & 1)) || (sj < P2 && (sj & 1))) return INFINITY;   // not a cluster representative
+    if ((si & ~1) == msk || (sj & ~1) == msk) return INFINITY;               // Sx is still being summed by k_chain
+    const int r = max(si, sj), c = min(si, sj);
+    const bool rowP = (r == si) == (i > j);                                  // the row holds the higher position
+    const double* Dr = D + (int64_t)r * ld;
+    double dpq;
+    if (r < P2) {
+        const double e0x = Dr[c], e0y = Dr[c + 1], e1x = Dr[ld + c], e1y = Dr[ld + c + 1];
+        dpq = (((e0x + (rowP ? e0y : e1x)) + (rowP ? e1x : e0y)) + e1y) * 0.25;
+    } else if (c < P2) {
+        dpq = (Dr[c] + Dr[c + 1]) * 0.5;
+    } else {
+        dpq = Dr[c];
+    }
+    const double Sr = Sx[r], Sc = Sx[c];
+    return (cm2 * dpq - (rowP ? Sr : Sc)) - (rowP ? Sc : Sr);
+}
+
+__global__ void __launch_bounds__(PRUNE_THREADS)
+k_prune(const double* __restrict__ D, int64_t ld, const double* __restrict__ Sx, const int* __restrict__ p2s,
+        const double* __restrict__ segmin, int64_t sld, const unsigned long long* __restrict__ smax, DevState* st,
+        const Partial* __restrict__ partials, int nseeds, unsigned short* __restrict__ chunk_mask, int min_m) {
+    const int m = st->m;
+    const bool on = min_m > 0 && !st->done && !(st->mode != 0 && m > st->fallback) && m >= min_m;
+    if (blockIdx.x == 0 && threadIdx.x == 0) st->prune_on = on;
+    if (!on) return;
+    const int P2 = st->P2, msk = st->mask_su, tid = threadIdx.x;
+    const double cm2 = (double)st->c - 2.0;
+    __shared__ double wmin[PRUNE_THREADS / 32];
+    double T = INFINITY;
+    for (int k = tid; k < nseeds; k += PRUNE_THREADS) {
+        const double q = seed_q(D, ld, Sx, p2s, m, P2, msk, cm2, partials[k].key);
+        T = q < T ? q : T;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) { const double o = __shfl_xor_sync(0xffffffffu, T, off); T = o < T ? o : T; }
+    if ((tid & 31) == 0) wmin[tid >> 5] = T;
+    __syncthreads();
+    for (int w = 0; w < PRUNE_THREADS / 32; ++w) T = wmin[w] < T ? wmin[w] : T;
+    const double delta = 16.0 * 1.1102230246251565e-16 * (3.0 * (double)st->c + 2.0) * st->Dmax
+                       + ((double)st->c + 2.0) * 4.9406564584124654e-324;
+    const double thr = T + 2.0 * delta;
+
+    unsigned long long kept = 0, skipped = 0;
+    // only the tiles this rank's scan owns (fnn_tile_iter.h: t = rank (mod world) while the scan is sharded)
+    const int ew = effective_world(st->world, m), first = ew > 1 ? st->rank : 0;
+    const long long total = tma::TileIter(m, 0, 1).total;
+    const long long nchunks = total > first ? 4 * ((total - first + ew - 1) / ew) : 0;
+    for (long long u = (long long)blockIdx.x * PRUNE_THREADS + tid; u < nchunks; u += (long long)gridDim.x * PRUNE_THREADS) {
+        const long long t = first + (long long)ew * (u / 4);
+        int r0, cb0;
+        tma::TileIter(m, (int)t, 1).decode(r0, cb0);
+        const int rc = r0 + (int)(u % 4) * tma::BOX_R;
+        unsigned bits = 0;
+        for (int i = 0; i < tma::BOX_R && rc + i < m; ++i) {
+            const int r = rc + i;
+            const bool pr = r < P2;
+            if (pr && (r & 1)) continue;   // decided with its even row
+            const bool masked = (r & ~1) == msk;
+            const double Sr = masked ? 0.0 : Sx[r];
+            for (int bx = 0; bx < 2; ++bx) {
+                const int cs = cb0 + bx * tma::BOX_W;
+                if (cs >= r || cs >= m) continue;   // no pair of this row in the segment
+                bool keep = false;
+                if (!masked) {   // the masked cluster's pairs are k_patch's
+                    const int b = cs / SEG;
+                    double sm = segmin[(int64_t)r * sld + b];
+                    if (pr) { const double s1 = segmin[(int64_t)(r + 1) * sld + b]; sm = (s1 < sm || s1 != s1) ? s1 : sm; }
+                    const double lb = (cm2 * sm - Sr) - ord_val(smax[b]);
+                    keep = !(lb > thr);
+                }
+                const int bit = bx * tma::BOX_R + i;
+                if (keep) bits |= (pr ? 3u : 1u) << bit;
+                else ++skipped;
+            }
+        }
+        chunk_mask[4 * t + u % 4] = (unsigned short)bits;
+        kept += (unsigned long long)__popc(bits) * (tma::BOX_W * 8);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        kept += __shfl_xor_sync(0xffffffffu, kept, off);
+        skipped += __shfl_xor_sync(0xffffffffu, skipped, off);
+    }
+    if ((tid & 31) == 0 && (kept || skipped)) { atomicAdd(&st->read_bytes, kept); atomicAdd(&st->units_skipped, skipped); }
+}
+
 // stand-alone entry for the exact left-to-right summation (parity tests of fnn_exact_sum.cuh)
 __global__ void __launch_bounds__(PICK_THREADS, 1)
 k_seqsum(const double* __restrict__ rows, int64_t stride, int nrows, int len, double* out, int serial_chain) {
@@ -967,12 +1139,21 @@ struct fnn_ctx {
     int chain_stage_cap = 0;          // elements of the chain that fit in shared memory (0: read from global)
     bool overlap = false;
     int force_exact = 0;              // A/B: always decide the pick with the exact left-to-right sums
+    // pruning of the selection scan (k_prune): segment minima per slot, segment maxima of Sx, survivor masks per tile chunk
+    double* segmin = nullptr;
+    int64_t sld = 0;                  // segments per row: ceil(ld / 256)
+    unsigned long long* smax = nullptr;
+    unsigned short* chunk_mask = nullptr;
+    int prune = 1;                    // A/B: opts.reserved[0] = 1 scans every segment
+    int prune_min_m = PRUNE_MIN_M;    // FNN_PRUNE_MIN_M overrides it for measuring the threshold
+    int64_t stop_after = 0;           // fnn_ctx_prune_bounds: run only this many iterations, launch by launch
+    int prune_grid = 0;
     cudaStream_t stream2 = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     bool join_pending = false;        // a k_chain + k_patch has been issued on stream2 and not yet waited for
-    int launches_per_iter() const { return 7 + (o.mode >= FNN_RANDOM_N ? 2 : 0) + (o.mode == FNN_RELAXED ? 1 : 0); }
+    int launches_per_iter() const { return 8 + (o.mode >= FNN_RANDOM_N ? 2 : 0) + (o.mode == FNN_RELAXED ? 1 : 0); }
     DevState* h_st = nullptr;  // pinned
-    CUtensorMap tmap;
+    CUtensorMap tmap, tmap_row;       // 8 x 256 and 1 x 256 boxes of the matrix
     bool have_tmap = false;
     int rank = 0, world = 1;
     long long run_counter = 0;
@@ -1037,6 +1218,7 @@ extern "C" void fnn_ctx_destroy(fnn_ctx* c) {
     cudaFree(c->nbrpos); cudaFree(c->pairs); cudaFree(c->walk); cudaFree(c->walk_ticket);
     cudaFree(c->id); cudaFree(c->pos); cudaFree(c->p2s); cudaFree(c->amalg); cudaFree(c->st); cudaFree(c->partials);
     cudaFree(c->rx_part); cudaFree(c->patch_part); cudaFree(c->tl);
+    cudaFree(c->segmin); cudaFree(c->smax); cudaFree(c->chunk_mask);
     if (c->h_st) cudaFreeHost(c->h_st);
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_join) cudaEventDestroy(c->ev_join);
@@ -1112,6 +1294,13 @@ static int ctx_build(fnn_ctx* c, const fnn_opts* o, int64_t n) {
     FNN_ALLOC(c->partials, sizeof(Partial) * c->partials_cap);
     FNN_ALLOC(c->rx_part, sizeof(double) * 8 * RX_BLOCKS_MAX);
     FNN_ALLOC(c->patch_part, sizeof(Partial) * PATCH_BLOCKS);
+    c->prune = o->reserved[0] == 1 ? 0 : 1;
+    if (const char* e = getenv("FNN_PRUNE_MIN_M")) c->prune_min_m = std::max(1, atoi(e));   // measurement aid only
+    c->sld = (c->ld + SEG - 1) / SEG;
+    c->prune_grid = 2 * c->sms;
+    FNN_ALLOC(c->segmin, sizeof(double) * n * c->sld);
+    FNN_ALLOC(c->smax, sizeof(unsigned long long) * c->sld);
+    FNN_ALLOC(c->chunk_mask, sizeof(unsigned long long) * std::max<long long>(1, tma::TileIter((int)n, 0, 1).total));
     if (o->record_trace) {
         FNN_ALLOC(c->trace, sizeof(double) * 8 * (n + 8));
         FNN_ALLOC(c->record, sizeof(long long) * rec::COLS * (n + 8));
@@ -1245,11 +1434,14 @@ static inline int check_partials(fnn_ctx* c, int grid, const char* kernel) {
 
 static inline int launch_scan(fnn_ctx* c) {
     if (int rc = check_partials(c, c->scan_grid, "k_scan_tma")) return rc;
-    tma::k_scan_tma<<<c->scan_grid, tma::THREADS, tma::SMEM_BYTES, c->stream>>>(c->tmap, c->Sx, c->pos, c->st, c->partials, c->peers);
+    k_prune<<<c->prune_grid, PRUNE_THREADS, 0, c->stream>>>(c->D, c->ld, c->Sx, c->p2s, c->segmin, c->sld, c->smax, c->st, c->partials,
+                                                          c->scan_grid, c->chunk_mask, c->prune ? c->prune_min_m : 0);
+    tma::k_scan_tma<<<c->scan_grid, tma::THREADS, tma::SMEM_BYTES, c->stream>>>(
+        c->tmap, c->tmap_row, c->Sx, c->pos, reinterpret_cast<const unsigned long long*>(c->chunk_mask), c->st, c->partials, c->peers);
     return FNN_OK;
 }
 
-// 2-D tiled tensor map over the n x ld matrix: box = 256 columns x 8 rows, no swizzle, zero OOB fill
+// 2-D tiled tensor maps over the n x ld matrix: boxes of 256 columns x 8 rows and x 1 row, no swizzle, zero OOB fill
 static int make_tensor_map(fnn_ctx* c) {
     typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -1260,12 +1452,14 @@ static int make_tensor_map(fnn_ctx* c) {
     if (!fn || qres != cudaDriverEntryPointSuccess) { fnn::set_error("cuTensorMapEncodeTiled not available"); return FNN_E_CUDA; }
     cuuint64_t gdim[2] = {(cuuint64_t)c->ld, (cuuint64_t)c->n};
     cuuint64_t gstr[1] = {(cuuint64_t)c->ld * sizeof(double)};
-    cuuint32_t box[2] = {(cuuint32_t)tma::BOX_W, (cuuint32_t)tma::BOX_R};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = ((EncodeFn)fn)(&c->tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, c->D, gdim, gstr, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { fnn::set_error("cuTensorMapEncodeTiled failed: %d", (int)r); return FNN_E_CUDA; }
+    for (int k = 0; k < 2; ++k) {
+        cuuint32_t box[2] = {(cuuint32_t)tma::BOX_W, k ? 1u : (cuuint32_t)tma::BOX_R};
+        CUresult r = ((EncodeFn)fn)(k ? &c->tmap_row : &c->tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, c->D, gdim, gstr, box, estr,
+                                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) { fnn::set_error("cuTensorMapEncodeTiled failed: %d", (int)r); return FNN_E_CUDA; }
+    }
     c->have_tmap = true;
     return FNN_OK;
 }
@@ -1286,8 +1480,9 @@ static inline int launch_rest(fnn_ctx* c) {
     k_rx_stage<<<c->row_grid, 256, 0, c->stream>>>(c->D, c->ld, c->id, c->pos, c->p2s, c->st, c->mail, c->rxs, c->rxs_ld, c->rx_part);
     k_pick<<<1, PICK_THREADS, PICK_SMEM, c->stream>>>(c->D, c->ld, c->Sx, c->id, c->pos, c->p2s, c->st, c->amalg, c->trace,
                                                     c->serial_chain, c->rxs, c->rxs_ld, c->rx_part, c->row_grid, c->force_exact);
-    k_rows<<<c->row_grid, 256, 0, c->stream>>>(c->D, c->ld, c->Sx, c->st, c->scratch);
-    k_scatter<<<c->row_grid, 256, 0, c->stream>>>(c->D, c->ld, c->Sx, c->pos, c->st, c->scratch, c->stage, c->id, c->p2s);
+    k_rows<<<c->row_grid, 256, 0, c->stream>>>(c->D, c->ld, c->Sx, c->st, c->scratch, c->smax);
+    k_scatter<<<c->row_grid, 256, 0, c->stream>>>(c->D, c->ld, c->Sx, c->pos, c->st, c->scratch, c->stage, c->id, c->p2s,
+                                                  c->segmin, c->sld, c->smax);
     cudaStream_t cs = c->stream;
     if (c->overlap) {
         cudaEventRecord(c->ev_fork, c->stream);
@@ -1353,12 +1548,13 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
     k_init_nodes<<<(ni + 255) / 256, 256, 0, c->stream>>>(ni, c->id, c->pos, c->p2s, c->st, c->o.mode, c->o.mult,
                                                           c->o.canonical_fallback, (long long)c->o.seed, c->rank, c->world, (long long)(++c->run_counter) << 32,
                                                           c->tl, c->tl_iter0, c->tl_count);
-    k_rowsum<<<(ni + 127) / 128, 128, 0, c->stream>>>(c->D, c->ld, ni, c->Sx, c->st);
+    FNN_CUDA(cudaMemsetAsync(c->smax, 0, sizeof(unsigned long long) * c->sld, c->stream));
+    k_rowsum<<<(ni + 127) / 128, 128, 0, c->stream>>>(c->D, c->ld, ni, c->Sx, c->st, c->segmin, c->sld, c->smax);
     FNN_CUDA(cudaGetLastError());
     // iterations in which no strategy runs keep a zero record row; the strategy kernels fill the others
     if (c->record) FNN_CUDA(cudaMemsetAsync(c->record, 0, sizeof(long long) * rec::COLS * (n + 8), c->stream));
     int64_t launches = 2, scans = 0;
-    const int64_t max_iters = n;  // n-3 .. n-1 iterations; kernels no-op once done
+    const int64_t max_iters = c->stop_after > 0 ? c->stop_after : n;  // n-3 .. n-1 iterations; kernels no-op once done
     double prof_ms = 0.0, prof_bytes = 0.0;
     int64_t prof_samples = 0;
 
@@ -1405,7 +1601,7 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
         }
         join_branch(c);
         FNN_CUDA(cudaGetLastError());
-    } else if (c->o.use_graph) {
+    } else if (c->o.use_graph && c->stop_after == 0) {
         constexpr int GI = 32;  // iterations per graph
         if (!c->graph) {
             cudaGraph_t g;
@@ -1437,7 +1633,7 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
             const bool strategy_only = c->graph_strategy && (m_known - 2 * batch * GI > (int64_t)c->o.canonical_fallback);
             for (int64_t b = 0; b < batch && it < max_iters; ++b, it += GI) {
                 FNN_CUDA(cudaGraphLaunch(strategy_only ? c->graph_strategy : c->graph, c->stream));
-                launches += (int64_t)(c->launches_per_iter() - (strategy_only ? 1 : 0)) * GI;
+                launches += (int64_t)(c->launches_per_iter() - (strategy_only ? 2 : 0)) * GI;
                 if (!strategy_only) scans += GI;
             }
             FNN_CUDA(cudaMemcpyAsync(c->h_st, c->st, sizeof(DevState), cudaMemcpyDeviceToHost, c->stream));
@@ -1461,6 +1657,11 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
         }
     }
     join_branch(c);
+    if (c->stop_after > 0) {   // a prefix of the run for fnn_ctx_prune_bounds: the state is read, there is no ordering
+        FNN_CUDA(cudaStreamSynchronize(c->stream));
+        FNN_CUDA(cudaStreamSynchronize(c->stream2));
+        return FNN_OK;
+    }
     FNN_CUDA(cudaMemcpyAsync(c->h_st, c->st, sizeof(DevState), cudaMemcpyDeviceToHost, c->stream));
     FNN_CUDA(cudaEventRecord(e1, c->stream));
     FNN_CUDA(cudaStreamSynchronize(c->stream));
@@ -1512,7 +1713,32 @@ extern "C" int fnn_ctx_order(fnn_ctx* c, int32_t* ordering) {
     c->stats.reserved[1] = (double)c->h_st->cert_fail;   // picks that needed the exact left-to-right sums
     c->stats.reserved[2] = (double)c->h_st->strat_bytes; // Relaxed row scans / Random samples: algorithmic bytes (SURVEY 8d K7/K9)
     c->stats.reserved[3] = (double)c->h_st->strat_units; // ... and their number
+    c->stats.reserved[4] = (double)c->h_st->read_bytes;  // matrix bytes the selection scan fetched (k_prune)
+    c->stats.reserved[5] = (double)c->h_st->units_skipped;   // row segments it did not fetch
     c->trace_rows = c->h_st->iter;
+    return FNN_OK;
+}
+
+extern "C" int fnn_ctx_prune_bounds(fnn_ctx* c, int64_t iters, double* D_out, double* segmin_out, uint64_t* smax_out,
+                                    double* Sx_out, int64_t* meta_out) {
+    if (!c || iters < 1 || !D_out || !segmin_out || !smax_out || !Sx_out || !meta_out || c->n <= 3) {
+        fnn::set_error("fnn_ctx_prune_bounds: bad arguments");
+        return FNN_E_ARG;
+    }
+    std::vector<int32_t> unused(c->n + 1);
+    c->stop_after = iters;
+    const int rc = fnn_ctx_order(c, unused.data());
+    c->stop_after = 0;
+    if (rc) return rc;
+    const int64_t n = c->n;
+    FNN_CUDA(cudaMemcpy2D(D_out, n * sizeof(double), c->D, c->ld * sizeof(double), n * sizeof(double), n, cudaMemcpyDeviceToHost));
+    FNN_CUDA(cudaMemcpy(segmin_out, c->segmin, sizeof(double) * n * c->sld, cudaMemcpyDeviceToHost));
+    FNN_CUDA(cudaMemcpy(smax_out, c->smax, sizeof(uint64_t) * c->sld, cudaMemcpyDeviceToHost));
+    FNN_CUDA(cudaMemcpy(Sx_out, c->Sx, sizeof(double) * n, cudaMemcpyDeviceToHost));
+    DevState h;
+    FNN_CUDA(cudaMemcpy(&h, c->st, sizeof(DevState), cudaMemcpyDeviceToHost));
+    meta_out[0] = h.m; meta_out[1] = h.P2; meta_out[2] = h.mask_su; meta_out[3] = h.iter; meta_out[4] = c->sld;
+    meta_out[5] = h.done;
     return FNN_OK;
 }
 
@@ -1550,7 +1776,7 @@ extern "C" int fnn_rowsums(const fnn_opts* o, const double* Dh, int64_t n, doubl
     if (rc) return rc;
     rc = fnn_ctx_load_host(c, Dh);
     if (!rc) {
-        k_rowsum<<<((int)n + 127) / 128, 128, 0, c->stream>>>(c->D, c->ld, (int)n, c->Sx, nullptr);
+        k_rowsum<<<((int)n + 127) / 128, 128, 0, c->stream>>>(c->D, c->ld, (int)n, c->Sx, nullptr, nullptr, 0, nullptr);
         if (cudaMemcpyAsync(Sx_out, c->Sx, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
             cudaStreamSynchronize(c->stream) != cudaSuccess) {
             fnn::set_error("fnn_rowsums: %s", cudaGetErrorString(cudaGetLastError()));

@@ -5,7 +5,10 @@
 // (6 x 32 KB), completion signalled through mbarriers; eight consumer warps evaluate
 // Q = (c-2)*Dpq - Sx[p] - Sx[q] on the staged rows and keep a per-thread (Q, i, j) min-loc.
 // Memory-level parallelism comes from the ring (up to 192 KB in flight per SM), not from
-// registers or occupancy.  Included by fnn_order.cu (needs DevState, Partial, better()).
+// registers or occupancy.  From 4 096 active nodes up, k_prune (fnn_order.cu) first marks the row segments (one row, or one
+// pair row, x 256 columns) whose lower bound on Q exceeds a Q already reached by a real pair; the scan then fetches only the
+// surviving segments (1 x 256 boxes, or the two 8 x 256 boxes when a whole chunk survives) and reads the others' rows as
+// Sx = -inf.  Included by fnn_order.cu (needs DevState, Partial, better()).
 #pragma once
 #include <cuda.h>
 #include "fnn_tile_iter.h"
@@ -174,14 +177,15 @@ __device__ __forceinline__ void eval_pp(const double* sm, const RowData* rd, dou
 }
 
 __global__ void __launch_bounds__(THREADS, 1)
-k_scan_tma(const __grid_constant__ CUtensorMap tmap, const double* __restrict__ Sx, const int* __restrict__ pos,
-           DevState* st, Partial* partials, const PeerTable* peers) {
+k_scan_tma(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_row, const double* __restrict__ Sx,
+           const int* __restrict__ pos, const unsigned long long* __restrict__ tile_mask, DevState* st, Partial* partials,
+           const PeerTable* peers) {
     if (st->done || (st->mode != 0 && st->m > st->fallback)) return;   // NetMakerOriginal.java:361-366
     extern __shared__ __align__(1024) unsigned char smem[];
     // keep the ring pointer in the shared window (no generic-address loads): offset, not integer cast
     double* ring = reinterpret_cast<double*>(smem + ((1024u - (smem_u32(smem) & 1023u)) & 1023u));
     __shared__ uint64_t full_bar[STAGES], empty_bar[STAGES];
-    __shared__ RowData rowdata[2][TILE_ROWS];
+    __shared__ RowData rowdata[2][2][TILE_ROWS];   // [tile parity][box][row]: S = -inf where the row segment is not fetched
     __shared__ Partial wbest[THREADS / 32];
     __shared__ bool amLast;
 
@@ -192,6 +196,11 @@ k_scan_tma(const __grid_constant__ CUtensorMap tmap, const double* __restrict__ 
     // the cluster created by the previous iteration: its u.Sx is still being summed by k_chain on a forked
     // branch, which also evaluates that cluster's pairs exactly; here its Sx reads as -inf, i.e. Q = +inf
     const int msk = st->mask_su;
+    // k_prune's survivor masks (one 64-bit word per tile: bit 16*chunk + 8*box + row) when it pruned this launch, else all ones
+    const bool pruned = st->prune_on;
+    const int tfirst = (ew > 1 ? st->rank : 0) + ew * blockIdx.x, tstride = ew * gridDim.x;
+    const long long ttotal = TileIter(m, 0, 1).total;
+    const int lane = tid & 31;
 
     if (tid == 0) {
         if (blockIdx.x == 0) tl_stamp(st, TL_SCAN0);
@@ -215,22 +224,42 @@ k_scan_tma(const __grid_constant__ CUtensorMap tmap, const double* __restrict__ 
     double bqd = INFINITY;
 
     if (tid >= CONSUMERS) {
-        // ===================== producer warp: one lane issues the TMA loads =====================
-        if (tid == CONSUMERS) {
-            int stage = 0;
-            uint32_t phase = 0;
-            for (TileIter it(m, (ew > 1 ? st->rank : 0) + ew * blockIdx.x, ew * gridDim.x); it.valid(); it.next()) {
+        // ===================== producer warp: issues the TMA loads of every chunk that holds a surviving row segment
+        // A chunk whose 16 row segments all survive is fetched as the two 8 x 256 boxes; otherwise each surviving segment is
+        // one 1 x 256 box (a pair row is two of them), and a chunk without survivors takes no stage at all.
+        int stage = 0;
+        uint32_t phase = 0;
+        for (long long w = tfirst; w < ttotal; w += 32LL * tstride) {
+            const long long tl = w + (long long)lane * tstride;
+            const unsigned long long mk = tl < ttotal ? (pruned ? tile_mask[tl] : ~0ull) : 0ull;
+            for (unsigned live = __ballot_sync(0xffffffffu, mk != 0); live; live &= live - 1) {
+                const int src = __ffs(live) - 1;
+                const unsigned long long tm = __shfl_sync(0xffffffffu, mk, src);
                 int r0, cb0;
-                it.decode(r0, cb0);
+                TileIter(m, (int)(w + (long long)src * tstride), 1).decode(r0, cb0);
                 const int rEnd = min(r0 + TILE_ROWS, m);
-                for (int rc = r0; rc < rEnd; rc += BOX_R) {
+                for (int ch = 0, rc = r0; rc < rEnd; ++ch, rc += BOX_R) {
+                    const unsigned cm = (unsigned)(tm >> (16 * ch)) & 0xffffu;
+                    if (!cm) continue;
                     const int rcEnd = min(rc + BOX_R, rEnd);
-                    mbar_wait(&empty_bar[stage], phase ^ 1);
-                    const bool second = (cb0 + BOX_W < rcEnd - 1) && (cb0 + BOX_W < m);
-                    mbar_expect_tx(&full_bar[stage], second ? STAGE_BYTES : STAGE_BYTES / 2);
                     double* dst = ring + (size_t)stage * (STAGE_BYTES / 8);
-                    tma_load_2d(dst, &tmap, cb0, rc, &full_bar[stage]);
-                    if (second) tma_load_2d(dst + BOX_R * BOX_W, &tmap, cb0 + BOX_W, rc, &full_bar[stage]);
+                    if (lane == 0) mbar_wait(&empty_bar[stage], phase ^ 1);
+                    if (cm == 0xffffu) {
+                        if (lane == 0) {
+                            const bool second = (cb0 + BOX_W < rcEnd - 1) && (cb0 + BOX_W < m);
+                            mbar_expect_tx(&full_bar[stage], second ? STAGE_BYTES : STAGE_BYTES / 2);
+                            tma_load_2d(dst, &tmap, cb0, rc, &full_bar[stage]);
+                            if (second) tma_load_2d(dst + BOX_R * BOX_W, &tmap, cb0 + BOX_W, rc, &full_bar[stage]);
+                        }
+                    } else {
+                        if (lane == 0) mbar_expect_tx(&full_bar[stage], (uint32_t)__popc(cm) * (BOX_W * 8));
+                        __syncwarp();
+                        if (lane < 2 * BOX_R && ((cm >> lane) & 1u)) {
+                            const int bx = lane / BOX_R, u = lane % BOX_R;
+                            tma_load_2d(dst + bx * (BOX_R * BOX_W) + u * BOX_W, &tmap_row, cb0 + bx * BOX_W, rc + u, &full_bar[stage]);
+                        }
+                    }
+                    __syncwarp();
                     if (++stage == STAGES) { stage = 0; phase ^= 1; }
                 }
             }
@@ -243,13 +272,20 @@ k_scan_tma(const __grid_constant__ CUtensorMap tmap, const double* __restrict__ 
         const int box = gt >> 7, lc = (gt & 127) * 2;   // which box of the stage, local column
         const int uo = grp * RPG;                       // first chunk row of this group
         int tileParity = 0;
-        for (TileIter it(m, (ew > 1 ? st->rank : 0) + ew * blockIdx.x, ew * gridDim.x); it.valid(); it.next(), tileParity ^= 1) {
+        for (long long w = tfirst; w < ttotal; w += 32LL * tstride) {   // the producer's tile sequence and masks
+          const long long tl = w + (long long)lane * tstride;
+          const unsigned long long mk = tl < ttotal ? (pruned ? tile_mask[tl] : ~0ull) : 0ull;
+          for (unsigned live = __ballot_sync(0xffffffffu, mk != 0); live; live &= live - 1, tileParity ^= 1) {
+            const int src = __ffs(live) - 1;
+            const unsigned long long tm = __shfl_sync(0xffffffffu, mk, src);
             int r0, cb0;
-            it.decode(r0, cb0);
+            TileIter(m, (int)(w + (long long)src * tstride), 1).decode(r0, cb0);
             const int rEnd = min(r0 + TILE_ROWS, m);
-            if (tid < TILE_ROWS && r0 + tid < m) {   // stage the tile's row data
-                rowdata[tileParity][tid].S = (((r0 + tid) & ~1) == msk) ? -INFINITY : Sx[r0 + tid];
-                rowdata[tileParity][tid].pos = pos[r0 + tid];
+            if (tid < 2 * TILE_ROWS && r0 + (tid % TILE_ROWS) < m) {   // stage the tile's row data, per box
+                const int bx = tid / TILE_ROWS, i = tid % TILE_ROWS, r = r0 + i;
+                const bool fetched = (tm >> (16 * (i / BOX_R) + BOX_R * bx + i % BOX_R)) & 1ull;
+                rowdata[tileParity][bx][i].S = ((r & ~1) == msk || !fetched) ? -INFINITY : Sx[r];
+                rowdata[tileParity][bx][i].pos = pos[r];
             }
             const int c0 = cb0 + box * BOX_W + lc;
             const bool cvalid = (c0 < m) && (c0 < rEnd - 1);   // some row of the tile lies strictly below column c0
@@ -263,12 +299,13 @@ k_scan_tma(const __grid_constant__ CUtensorMap tmap, const double* __restrict__ 
             }
             asm volatile("bar.sync 1, %0;" ::"n"(CONSUMERS) : "memory");
 
-            for (int rc = r0; rc < rEnd; rc += BOX_R) {
+            for (int ch = 0, rc = r0; rc < rEnd; ++ch, rc += BOX_R) {
+                if (!((tm >> (16 * ch)) & 0xffffull)) continue;   // no surviving row segment: nothing was fetched
                 const int rcEnd = min(rc + BOX_R, rEnd);
                 mbar_wait(&full_bar[stage], phase);
                 const double* sm = ring + (size_t)stage * (STAGE_BYTES / 8) + box * (BOX_R * BOX_W) + lc + uo * BOX_W;
                 const int ra = rc + uo, rb = min(ra + RPG, rcEnd);   // this group's rows of the chunk
-                const RowData* rd = &rowdata[tileParity][ra - r0];
+                const RowData* rd = &rowdata[tileParity][box][ra - r0];
                 if (cvalid && c0 < rb - 1) {
                     const bool full_rows = (rcEnd - rc == BOX_R);
                     if (colPair && full_rows && rcEnd <= P2 && c0 < ra) {
@@ -331,6 +368,7 @@ k_scan_tma(const __grid_constant__ CUtensorMap tmap, const double* __restrict__ 
                 if ((tid & 31) == 0) mbar_arrive(&empty_bar[stage]);
                 if (++stage == STAGES) { stage = 0; phase ^= 1; }
             }
+          }
         }
     }
 

@@ -60,7 +60,8 @@ typedef struct fnn_opts {
     int32_t use_graph;          /* 1: replay the per-iteration kernel sequence as a CUDA graph */
     int32_t record_trace;       /* 1: keep the per-iteration (m,c,Cx,Cy,x,y,kind,best) trace on device */
     int32_t profile_every;      /* >0: time the selection kernel of every k-th iteration with CUDA events */
-    int32_t reserved[6];        /* A/B switches, 0 = production: [1]=1: sum the sequential chains on one lane instead of the
+    int32_t reserved[6];        /* A/B switches, 0 = production: [0]=1: the selection scan reads every row segment (no
+                                   lower-bound pruning, DESIGN.md §4.1); [1]=1: sum the sequential chains on one lane instead of the
                                    collapsed exact summation; [3]=1: split weights = unconstrained closed form only;
                                    [4]: split-weight solver variant (see fnn_split_weights); [5] bit 0: u.Sx chain on the
                                    critical path instead of the forked branch, bit 1: always decide the 4-candidate pick
@@ -80,7 +81,10 @@ typedef struct fnn_stats {
     double order_ms;           /* device time of the whole ordering run (CUDA events) */
     double h2d_ms;             /* device time of the host->device matrix upload, if any */
     double reserved[8];        /* [0] 4-candidate picks decided by the certified parallel ComputeRx sums, [1] picks that
-                                  needed the exact left-to-right sums (NetMakerOriginal.java:413-452) */
+                                  needed the exact left-to-right sums (NetMakerOriginal.java:413-452), [2] [3] Relaxed / Random
+                                  algorithmic bytes and units, [4] matrix bytes the selection scan fetched (pruned launches:
+                                  the surviving row segments; others: their algorithmic bytes), [5] row segments (a pair row
+                                  counts once) that pruned launches skipped */
 } fnn_stats;
 
 void fnn_default_opts(fnn_opts* o);
@@ -121,6 +125,13 @@ int64_t fnn_ctx_trace(fnn_ctx* c, double* rows_out, int64_t max_rows);
  * The digest (a uint64 stored as int64) is defined in csrc/fnn_record.h; a test hook for holding the strategies to a CPU
  * restatement draw for draw. */
 int64_t fnn_ctx_strategy_record(fnn_ctx* c, int64_t* rows_out, int64_t max_rows);
+/* Test hook of the selection scan's pruning bounds (DESIGN.md §4.1): runs the first `iters` iterations of fnn_ctx_order on
+ * the loaded matrix (which it consumes) and returns the device state after them: D_out[n*n] (slot layout), the segment
+ * minima segmin_out[n * S] (S = meta_out[4] segments of 256 columns per slot), the segment maxima of Sx smax_out[S] as
+ * order-preserving keys (k >> 63 ? k ^ 2^63 : ~k are the double's bits; 0 = none), Sx_out[n], and meta_out[6] =
+ * {m, P2, masked cluster's base slot or -1, iterations done, S, done}. */
+int fnn_ctx_prune_bounds(fnn_ctx* c, int64_t iters, double* D_out, double* segmin_out, uint64_t* smax_out, double* Sx_out,
+                         int64_t* meta_out);
 int fnn_ctx_stats(fnn_ctx* c, fnn_stats* out);
 /* device pointer + leading dimension of the internal matrix (for zero-copy producers such as torch) */
 int fnn_ctx_matrix_ptr(fnn_ctx* c, double** dptr, int64_t* ld);

@@ -23,4 +23,6 @@ for n in [int(a) for a in args] or [5000, 20000]:
             s = c.stats()
             print(f"n={n} mode={mode} eps={eps} opts={opts} wall={dt:.3f}s dev={s['order_ms']/1e3:.3f}s iterations={s['iterations']} "
                   f"launches={s['kernel_launches']} alg={s['scan_alg_bytes']/dt/1e9:.0f} GB/s certified={s['picks_certified']} "
-                  f"exact={s['picks_exact']} strat_units={s['strategy_units']} sha={hashlib.sha256(o.tobytes()).hexdigest()[:16]}", flush=True)
+                  f"exact={s['picks_exact']} strat_units={s['strategy_units']} read={s['scan_read_bytes']/1e9:.1f} GB "
+                  f"of alg={s['scan_alg_bytes']/1e9:.1f} GB skipped_units={s['scan_units_skipped']} "
+                  f"sha={hashlib.sha256(o.tobytes()).hexdigest()[:16]}", flush=True)
