@@ -25,6 +25,9 @@ from .api import (  # noqa: F401
     network_splits,
     network,
     read_phylip,
+    read_alignment,
+    distances,
+    MODELS,
     write_nexus,
     java_double_str,
     release_cache,

@@ -1,7 +1,8 @@
-"""`python -m fastneighbornet_b200 -distFile in.phy [...]` — the run of FastNN.main (FastNN.java:113-480) over libfastnn.so.
+"""`python -m fastneighbornet_b200 -distFile in.phy | -seqFile aln.fa [...]` — the run of FastNN.main (FastNN.java:113-480) over libfastnn.so.
 
 A thin driver, kept only so that the three native stages can be exercised the way the reference is invoked:
 fnn_read_phylip -> fnn_network (ordering, split weights, kept splits; distances stay on the device) -> fnn_write_nexus.
+-seqFile replaces the first stage with fnn_read_alignment -> fnn_distances (--distance p|jc69|k2p, --undefined VALUE).
 Options carry the reference's names (FastNN.java:130-172); -threads is accepted and only sizes the host-side loader and
 writer pools.  --seed is new: the reference draws from an unseedable ThreadLocalRandom in the Relaxed/Random modes.
 """
@@ -19,7 +20,10 @@ MODES = {"CANONICAL": "canonical", "RELAXED": "relaxed", "RANDOM_N": "random_n",
 def parse_args(argv):
     ap = argparse.ArgumentParser(prog="python -m fastneighbornet_b200", prefix_chars="-", allow_abbrev=False,
                                  description="Neighbor-Net on a B200: circular ordering and weighted splits as Nexus on stdout.")
-    ap.add_argument("-distFile", required=True, metavar="file_location", help="Phylip distance matrix (lower-triangular or square)")
+    src = ap.add_mutually_exclusive_group(required=True)
+    src.add_argument("-distFile", metavar="file_location", help="Phylip distance matrix (lower-triangular or square)")
+    src.add_argument("-seqFile", metavar="file_location",
+                     help="nucleotide alignment (FASTA or sequential PHYLIP); distances are computed on the GPU")
     ap.add_argument("-threads", type=int, default=0, metavar="integer", help="host threads for the loader/writer (0 = all)")
     ap.add_argument("-mode", default="CANONICAL", metavar="string", help="|".join(MODES))
     ap.add_argument("-mult", type=int, default=5, metavar="integer", help="multiplier of the Random_* sample sizes")
@@ -29,6 +33,9 @@ def parse_args(argv):
     ap.add_argument("--seed", type=int, default=12345)
     ap.add_argument("--no-distances", action="store_true", help="leave the n x n Distances block out of the Nexus output")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--distance", default="p", choices=list(api.MODELS), help="distance model of -seqFile (default p)")
+    ap.add_argument("--undefined", type=float, default=None, metavar="VALUE",
+                    help="-seqFile: distance of a pair with no comparable site or a saturated one (default: such a pair is an error)")
     a = ap.parse_args(argv)
     if a.mode.upper() not in MODES:
         ap.error(f"-mode must be one of {', '.join(MODES)}")
@@ -39,7 +46,11 @@ def parse_args(argv):
 def main(argv=None):
     a = parse_args(sys.argv[1:] if argv is None else argv)
     t0 = time.perf_counter()
-    D, names = api.read_phylip(a.distFile, threads=a.threads)
+    if a.seqFile:
+        codes, names = api.read_alignment(a.seqFile, threads=a.threads)
+        D = api.distances(codes, model=a.distance, undefined=a.undefined, device=a.device)
+    else:
+        D, names = api.read_phylip(a.distFile, threads=a.threads)
     n = D.shape[0]
     t1 = time.perf_counter()
     print(f"Calculating a network for {n} taxa on CUDA device {a.device}.", file=sys.stderr)

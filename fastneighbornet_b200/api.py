@@ -62,8 +62,11 @@ ABI_SYMBOLS = [
     "fnn_split_weights", "fnn_csw_matvec", "fnn_ctx_ipc_handle", "fnn_ctx_connect", "fnn_weighted_splits", "fnn_network",
     "fnn_phylip_taxa", "fnn_read_phylip", "fnn_write_nexus", "fnn_java_double_to_string", "fnn_release_cache",
     "fnn_ctx_load_host_rows", "fnn_ctx_commit_load", "fnn_split_weights_budget", "fnn_ctx_strategy_record",
-    "fnn_ctx_prune_bounds",
+    "fnn_ctx_prune_bounds", "fnn_alignment_size", "fnn_read_alignment", "fnn_ctx_load_alignment", "fnn_distances",
 ]
+
+# enum fnn_dist_model: distances from a nucleotide alignment (include/fastnn.h)
+MODELS = {"p": 0, "jc69": 1, "k2p": 2}
 
 
 def lib_path():
@@ -128,6 +131,13 @@ def lib():
                                   ctypes.POINTER(ctypes.c_int64)]
         L.fnn_csw_matvec.argtypes = [ctypes.POINTER(fnn_opts), ctypes.c_int32, c_dp, ctypes.c_int64, c_dp]
         L.fnn_seq_sum.argtypes = [ctypes.POINTER(fnn_opts), c_dp, ctypes.c_int32, ctypes.c_int64, c_dp]
+        c_bp = ctypes.POINTER(ctypes.c_uint8)
+        L.fnn_alignment_size.argtypes = [ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]
+        L.fnn_read_alignment.argtypes = [ctypes.c_char_p, ctypes.c_int64, ctypes.c_int64, c_bp, ctypes.c_char_p, ctypes.c_int64,
+                                         ctypes.c_int]
+        L.fnn_ctx_load_alignment.argtypes = [vp, c_bp, ctypes.c_int64, ctypes.c_int32, ctypes.c_double]
+        L.fnn_distances.argtypes = [ctypes.POINTER(fnn_opts), c_bp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int32, ctypes.c_double,
+                                    c_dp]
         _LIB = L
     return _LIB
 
@@ -165,6 +175,16 @@ def default_opts(**kw):
 
 def _dp(a):
     return a.ctypes.data_as(ctypes.POINTER(ctypes.c_double))
+
+
+def _alignment_args(codes, model, undefined):
+    """codes as a C-contiguous uint8 [n, L] array, the model's enum value and undefined_value (None -> NaN: fail)."""
+    codes = np.ascontiguousarray(codes, dtype=np.uint8)
+    if codes.ndim != 2:
+        raise ValueError("codes must be a 2-D [taxa, sites] array")
+    if model not in MODELS:
+        raise ValueError(f"model must be one of {', '.join(MODELS)}")
+    return codes, MODELS[model], float("nan") if undefined is None else float(undefined)
 
 
 class Context:
@@ -249,6 +269,13 @@ class Context:
         _check(lib().fnn_ctx_synth(self._h, _dp(h), _dp(a), inv.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
                                    ctypes.c_uint64(_s.stream_base(seed, 3)), float(eps)))
 
+    def load_alignment(self, codes, model="p", undefined=None):
+        """Distances of an [n, L] code array (read_alignment) computed on the device into this context's matrix
+        (fnn_ctx_load_alignment).  undefined=None: an undefined pair is an error; a finite value >= 0 is stored there."""
+        codes, m, u = _alignment_args(codes, model, undefined)
+        assert codes.shape[0] == self.n
+        _check(lib().fnn_ctx_load_alignment(self._h, codes.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)), codes.shape[1], m, u))
+
     def read_matrix(self):
         out = np.empty((self.n, self.n), dtype=np.float64)
         _check(lib().fnn_ctx_read_matrix(self._h, _dp(out)))
@@ -329,6 +356,8 @@ class Context:
         out["strategy_units"] = int(s.reserved[3])
         out["scan_read_bytes"] = float(s.reserved[4])      # matrix bytes the selection scan fetched (pruned segments not)
         out["scan_units_skipped"] = int(s.reserved[5])     # row segments the pruned scans did not fetch
+        out["dist_pack_ms"] = float(s.reserved[6])         # load_alignment: bit-plane packing kernel (h2d_ms: the codes' upload)
+        out["dist_pairs_ms"] = float(s.reserved[7])        # load_alignment: pair kernel
         return out
 
 
@@ -437,6 +466,32 @@ def read_phylip(path, threads=0, name_len=64):
     _check(lib().fnn_read_phylip(str(path).encode(), n, _dp(D), names, name_len, int(threads)))
     raw = names.raw
     return D, [raw[i * name_len:(i + 1) * name_len].split(b"\0", 1)[0].decode("ascii", "replace") for i in range(n)]
+
+
+def read_alignment(path, threads=0, name_len=64):
+    """Native FASTA / sequential PHYLIP alignment loader (fnn_alignment_size + fnn_read_alignment; host only, no device
+    needed).  Returns (codes[n, L] uint8 with A=0 C=1 G=2 T=3 and 4 = missing, names list)."""
+    n, L = ctypes.c_int64(), ctypes.c_int64()
+    _check(lib().fnn_alignment_size(str(path).encode(), ctypes.byref(n), ctypes.byref(L)))
+    n, L = n.value, L.value
+    codes = np.empty((n, L), dtype=np.uint8)
+    names = ctypes.create_string_buffer(n * name_len)
+    _check(lib().fnn_read_alignment(str(path).encode(), n, L, codes.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)), names, name_len,
+                                    int(threads)))
+    raw = names.raw
+    return codes, [raw[i * name_len:(i + 1) * name_len].split(b"\0", 1)[0].decode("ascii", "replace") for i in range(n)]
+
+
+def distances(codes, model="p", undefined=None, **opts):
+    """fnn_distances: the [n, n] float64 distance matrix of an [n, L] code array, computed on the device.
+    model: "p" | "jc69" | "k2p"; undefined=None: an undefined pair (no comparable site, saturation) is an error naming the
+    first such pair; a finite value >= 0 is stored there instead."""
+    codes, m, u = _alignment_args(codes, model, undefined)
+    o = default_opts(**opts)
+    n, L = codes.shape
+    D = np.empty((n, n), dtype=np.float64)
+    _check(lib().fnn_distances(ctypes.byref(o), codes.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)), n, L, m, u, _dp(D)))
+    return D
 
 
 def java_double_str(v):

@@ -33,6 +33,8 @@ struct DevEvent {
 // internal accessors across translation units (not part of the ABI)
 int64_t fnn_ctx_n_(fnn_ctx* c);
 void fnn_ctx_mark_loaded_(fnn_ctx* c);
+void fnn_ctx_mark_unloaded_(fnn_ctx* c);
+fnn_stats* fnn_ctx_stats_(fnn_ctx* c);
 int fnn_ctx_device_(fnn_ctx* c);
 int fnn_ctx_sms_(fnn_ctx* c);
 cudaStream_t fnn_ctx_stream_(fnn_ctx* c);

@@ -1790,6 +1790,8 @@ extern "C" int fnn_rowsums(const fnn_opts* o, const double* Dh, int64_t n, doubl
 // internal accessors for the other translation units of the library (not part of the ABI)
 int64_t fnn_ctx_n_(fnn_ctx* c) { return c->n; }
 void fnn_ctx_mark_loaded_(fnn_ctx* c) { c->loaded = true; }
+void fnn_ctx_mark_unloaded_(fnn_ctx* c) { c->loaded = false; }
+fnn_stats* fnn_ctx_stats_(fnn_ctx* c) { return &c->stats; }
 int fnn_ctx_device_(fnn_ctx* c) { return c->o.device; }
 int fnn_ctx_sms_(fnn_ctx* c) { return c->sms; }
 cudaStream_t fnn_ctx_stream_(fnn_ctx* c) { return c->stream; }

@@ -117,3 +117,57 @@ def read_phylip(path):
             if row == n:
                 break
     return D, names
+
+
+# ---- nucleotide alignments (A=0 C=1 G=2 T=3, 4 = missing; the codes of api.read_alignment) ----------------------------
+
+def simulate_alignment(n, L, seed, rate=0.3, gap_frac=0.0, kappa=2.0):
+    """n x L uint8 alignment evolved under K2P along a random tree (seeded numpy).
+
+    The tree is a random recursive tree: taxon k > 0 descends from a uniformly drawn earlier taxon over a branch of length
+    Exp(1) * rate / max(1, ln n) substitutions per site, so a tip lies about `rate` substitutions from taxon 0 whatever n is
+    and pairs stay far from saturation for rate <= 0.5.  Along a branch of length t each site takes a transition with
+    probability 1/4 + e^(-4 b t)/4 - e^(-2 (a + b) t)/2 and one of the two transversions with probability 1/2 - e^(-4 b t)/2,
+    with a = kappa / (kappa + 2), b = 1 / (kappa + 2).  A fraction gap_frac of the entries, drawn uniformly, is then set
+    missing."""
+    rng = np.random.default_rng(seed)
+    codes = np.empty((n, L), dtype=np.uint8)
+    codes[0] = rng.integers(0, 4, L, dtype=np.uint8)
+    a, b = kappa / (kappa + 2.0), 1.0 / (kappa + 2.0)
+    scale = rate / max(1.0, float(np.log(n)))
+    parents = np.concatenate([[0], [int(rng.integers(0, k)) for k in range(1, n)]]) if n > 1 else np.zeros(1, dtype=np.int64)
+    lengths = rng.exponential(scale, n)
+    flip = np.array([1, 3], dtype=np.uint8)
+    for k in range(1, n):
+        t = lengths[k]
+        p_ts = 0.25 + 0.25 * np.exp(-4 * b * t) - 0.5 * np.exp(-2 * (a + b) * t)
+        p_tv = 0.5 - 0.5 * np.exp(-4 * b * t)
+        u = rng.random(L)
+        x = codes[parents[k]].copy()
+        ts = u < p_ts
+        tv = (u >= p_ts) & (u < p_ts + p_tv)
+        x[ts] ^= 2
+        x[tv] ^= flip[rng.integers(0, 2, int(tv.sum()))]
+        codes[k] = x
+    if gap_frac > 0:
+        codes[rng.random((n, L)) < gap_frac] = 4
+    return codes
+
+
+def write_alignment(path, codes, names=None, fmt="fasta", width=60):
+    """FASTA (sequences wrapped at `width`) or sequential relaxed PHYLIP (`n L`, then `name sequence` lines) of a code array;
+    missing data is written as '-'."""
+    n, L = codes.shape
+    letters = np.frombuffer(b"ACGT-", dtype=np.uint8)
+    with open(path, "w") as f:
+        if fmt == "phylip":
+            f.write(f"{n} {L}\n")
+        for i in range(n):
+            nm = names[i] if names is not None else f"t{i + 1}"
+            seq = letters[codes[i]].tobytes().decode()
+            if fmt == "phylip":
+                f.write(f"{nm} {seq}\n")
+            else:
+                f.write(f">{nm}\n")
+                for s in range(0, L, width):
+                    f.write(seq[s:s + width] + "\n")

@@ -223,6 +223,47 @@ int fnn_csw_matvec(const fnn_opts* o, int32_t which, const double* v, int64_t n,
 int fnn_split_weights_budget(const fnn_opts* o, const int32_t* ordering, const double* d_upper, int64_t n, int64_t max_cg_iters,
                              int64_t max_cg_calls, double* x_out, uint8_t* active_out, int64_t* stats_out);
 
+/* ---- distances from a nucleotide alignment ---------------------------------------------------
+ * An alignment is n taxa x L sites of codes, row-major uint8: A=0 C=1 G=2 T=3, 4 = missing.  The loader reads U as T and the
+ * IUPAC ambiguity letters R Y S W K M B D H V N, plus X - ?, as missing (case-insensitive).  For a pair (i, j), with pairwise
+ * deletion: v = sites where both hold a state, m = those of them where the states differ, s = transitions among the m
+ * (A<->G, C<->T), q = m - s transversions; 32-bit counts, so 1 <= L <= 2^31-1.  Binary64 without FMA, in this order:
+ *   FNN_DIST_P:    d = (double)m / (double)v
+ *   FNN_DIST_JC69: p = m / v;  d = -0.75 * fnn_log(1.0 - p / 0.75)
+ *   FNN_DIST_K2P:  P = s / v;  Q = q / v;  d = (-0.5 * fnn_log((1.0 - 2.0 * P) - Q)) - (0.25 * fnn_log(1.0 - 2.0 * Q))
+ * fnn_log (csrc/fnn_log.h) is a logarithm built from IEEE + - * / alone, so the device and the CPU oracle give the same
+ * bits; it is within 1 ulp of the correctly rounded log.  A result of -0.0 (m = 0) is stored as +0.0, the diagonal is +0.0
+ * and D[i][j], D[j][i] are the same bits.  A pair is undefined when v = 0 or an argument of a log is <= 0 (saturation):
+ *   undefined_value NaN:            the call fails with FNN_E_ARG, fnn_last_error() names the first undefined pair (i < j,
+ *                                   lowest i, then lowest j) with its v, m and s; a context is left unloaded;
+ *   undefined_value finite, >= 0:   every undefined entry gets that value;
+ *   anything else:                  FNN_E_ARG.
+ * So every matrix these calls return lies in the verified domain of the ordering (finite, non-negative, symmetric, zero
+ * diagonal).  A code above 4 is FNN_E_ARG.  The computation is deterministic: ranks of a multi-GPU run that load the same
+ * codes hold the same bits.  DESIGN.md §4.4. */
+enum fnn_dist_model {
+    FNN_DIST_P = 0,
+    FNN_DIST_JC69 = 1,
+    FNN_DIST_K2P = 2
+};
+/* Alignment loader (host only, needs no device).  The first non-blank byte picks the format: '>' (or ';') FASTA - the name is
+ * the header text up to the first whitespace, sequences may wrap over any number of lines, lines may end in CRLF, lines
+ * starting with ';' are skipped; a digit: sequential relaxed PHYLIP - first line `n L`, then n lines `name<whitespace>sequence`
+ * whose sequence has exactly L characters once whitespace is removed (interleaved PHYLIP is rejected).  Whitespace inside
+ * sequence lines is skipped.  FNN_E_IO, with a message naming the taxon or the line and column: unequal sequence lengths, an
+ * empty sequence, no sequences, a sequence count that does not match the PHYLIP header, a byte that is not a code.
+ * fnn_alignment_size: n and L (FASTA: L of the first record).  fnn_read_alignment: codes[n*sites]; names (optional) receives n
+ * NUL-terminated names name_stride bytes apart (truncated to fit), as fnn_read_phylip; threads 0 = all host cores. */
+int fnn_alignment_size(const char* path, int64_t* n_out, int64_t* sites_out);
+int fnn_read_alignment(const char* path, int64_t n, int64_t sites, uint8_t* codes, char* names, int64_t name_stride, int threads);
+/* Distances of the context's n taxa (codes: n*sites) computed on its device into its own matrix, then marked loaded as
+ * fnn_ctx_synth does; fnn_ctx_order consumes it like any other load.  fnn_ctx_stats afterwards: h2d_ms = upload of the codes,
+ * reserved[6] = packing kernel, reserved[7] = pair kernel (CUDA-event ms). */
+int fnn_ctx_load_alignment(fnn_ctx* c, const uint8_t* codes, int64_t sites, int32_t model, double undefined_value);
+/* Host in, host out: D_out (n*n, row-major) on device opts->device (o NULL = defaults); needs no context. */
+int fnn_distances(const fnn_opts* o, const uint8_t* codes, int64_t n, int64_t sites, int32_t model, double undefined_value,
+                  double* D_out);
+
 /* left-to-right fp64 sums of nrows (<=4) rows of length len, bit-identical to `for (i) s += x[i]`
  * (the accumulation order of ComputeRx / updateClusterDistances, NetMakerOriginal.java:549-561, :530-535),
  * computed by the parallel exact-summation kernel (csrc/fnn_exact_sum.cuh) - exposed for parity tests */
