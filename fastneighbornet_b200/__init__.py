@@ -24,6 +24,7 @@ from .api import (  # noqa: F401
     weighted_splits,
     network_splits,
     network,
+    bootstrap,
     read_phylip,
     read_alignment,
     distances,

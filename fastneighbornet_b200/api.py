@@ -7,6 +7,7 @@ Reference interface mirrored (argument meaning and error behaviour kept):
   int[] runNeighborNet()                                   (NetMakerOriginal.java:51,129)
 `nThreads`/`pool` are accepted and ignored (single host control thread; SURVEY §8b).
 """
+import collections
 import ctypes
 import os
 
@@ -63,6 +64,7 @@ ABI_SYMBOLS = [
     "fnn_phylip_taxa", "fnn_read_phylip", "fnn_write_nexus", "fnn_java_double_to_string", "fnn_release_cache",
     "fnn_ctx_load_host_rows", "fnn_ctx_commit_load", "fnn_split_weights_budget", "fnn_ctx_strategy_record",
     "fnn_ctx_prune_bounds", "fnn_alignment_size", "fnn_read_alignment", "fnn_ctx_load_alignment", "fnn_distances",
+    "fnn_write_nexus_support", "fnn_bootstrap",
 ]
 
 # enum fnn_dist_model: distances from a nucleotide alignment (include/fastnn.h)
@@ -125,6 +127,8 @@ def lib():
         ip32 = ctypes.POINTER(ctypes.c_int32)
         L.fnn_write_nexus.argtypes = [ctypes.c_char_p, ctypes.c_int64, ctypes.c_char_p, ctypes.c_int64, c_dp, ip32, ip32, ip32, c_dp,
                                       ctypes.c_int64, ctypes.c_int]
+        L.fnn_write_nexus_support.argtypes = [ctypes.c_char_p, ctypes.c_int64, ctypes.c_char_p, ctypes.c_int64, c_dp, ip32, ip32, ip32,
+                                              c_dp, ip32, ctypes.c_int32, ctypes.c_int64, ctypes.c_int]
         L.fnn_java_double_to_string.argtypes = [ctypes.c_double, ctypes.c_char_p, ctypes.c_int64]
         L.fnn_network.argtypes = [ctypes.POINTER(fnn_opts), c_dp, ctypes.c_int64, ctypes.c_double, ctypes.POINTER(ctypes.c_int32),
                                   ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32), c_dp, ctypes.c_int64,
@@ -138,6 +142,9 @@ def lib():
         L.fnn_ctx_load_alignment.argtypes = [vp, c_bp, ctypes.c_int64, ctypes.c_int32, ctypes.c_double]
         L.fnn_distances.argtypes = [ctypes.POINTER(fnn_opts), c_bp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int32, ctypes.c_double,
                                     c_dp]
+        L.fnn_bootstrap.argtypes = [ctypes.POINTER(fnn_opts), c_bp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int32, ctypes.c_double,
+                                    ctypes.c_int32, ctypes.c_int64, ctypes.c_double, ip32, ip32, ip32, c_dp, ip32, ctypes.c_int64,
+                                    ctypes.POINTER(ctypes.c_int64), ip32, ctypes.POINTER(ctypes.c_int64), c_dp]
         _LIB = L
     return _LIB
 
@@ -501,8 +508,12 @@ def java_double_str(v):
     return buf.value.decode()
 
 
-def write_nexus(path, ordering, split_i, split_j, weight, D=None, names=None, threads=0):
-    """fnn_write_nexus: the output of OutputPrinter.NexusWithSplitsAndDistances for the kept splits (host only)."""
+def write_nexus(path, ordering, split_i, split_j, weight, D=None, names=None, threads=0, support=None, replicates=None):
+    """fnn_write_nexus: the output of OutputPrinter.NexusWithSplitsAndDistances for the kept splits (host only).
+    support (with replicates): bootstrap support counts of the splits (bootstrap); every split line then carries the
+    confidence 100 * support / replicates (fnn_write_nexus_support)."""
+    if (support is None) != (replicates is None):
+        raise ValueError("support and replicates go together")
     ordering = np.ascontiguousarray(ordering, dtype=np.int32)
     n = ordering.shape[0] - 1
     si = np.ascontiguousarray(split_i, dtype=np.int32)
@@ -518,8 +529,16 @@ def write_nexus(path, ordering, split_i, split_j, weight, D=None, names=None, th
     if D is not None:
         D = np.ascontiguousarray(D, dtype=np.float64)
         Dp = _dp(D)
-    _check(lib().fnn_write_nexus(None if path is None else str(path).encode(), n, nbuf, stride, Dp, ordering.ctypes.data_as(ip),
-                                 si.ctypes.data_as(ip), sj.ctypes.data_as(ip), _dp(w), len(w), int(threads)))
+    if support is None:
+        _check(lib().fnn_write_nexus(None if path is None else str(path).encode(), n, nbuf, stride, Dp, ordering.ctypes.data_as(ip),
+                                     si.ctypes.data_as(ip), sj.ctypes.data_as(ip), _dp(w), len(w), int(threads)))
+        return
+    sup = np.ascontiguousarray(support, dtype=np.int32)
+    if sup.shape != w.shape:
+        raise ValueError("support needs one count per split")
+    _check(lib().fnn_write_nexus_support(None if path is None else str(path).encode(), n, nbuf, stride, Dp, ordering.ctypes.data_as(ip),
+                                         si.ctypes.data_as(ip), sj.ctypes.data_as(ip), _dp(w), sup.ctypes.data_as(ip), int(replicates),
+                                         len(w), int(threads)))
 
 
 def network(D, cutoff=1e-6, **opts):
@@ -537,6 +556,41 @@ def network(D, cutoff=1e-6, **opts):
                              sj.ctypes.data_as(ip), _dp(w), cap, ctypes.byref(kept)))
     k = kept.value
     return ordering, si[:k].copy(), sj[:k].copy(), w[:k].copy()
+
+
+Bootstrap = collections.namedtuple("Bootstrap", "ordering split_i split_j weight support replicate_kept replicate_orderings times")
+
+
+def bootstrap(codes, replicates, model="p", boot_seed=12345, undefined=None, cutoff=1e-6, replicate_orderings=False, **opts):
+    """fnn_bootstrap: the network of an [n, L] code array (as network(distances(codes))) and the bootstrap support of its
+    kept splits over `replicates` column resamplings drawn from java.util.Random(boot_seed), every replicate computed on the
+    device.  opts are the ordering options (mode, mult, seed, canonical_fallback, device); every replicate's ordering starts
+    from the same seed.  Returns a Bootstrap tuple: ordering, split_i, split_j, weight (the original network), support
+    (int32 per kept split, 0..replicates), replicate_kept (kept splits per replicate), replicate_orderings ([R, n+1] when
+    asked for, else None) and times (ms summed over the replicates: distances, ordering, split_weights, matching; and
+    cg_iters)."""
+    codes, m, u = _alignment_args(codes, model, undefined)
+    n, L = codes.shape
+    R = int(replicates)
+    o = default_opts(**opts)
+    cap = max(1, n * (n - 1) // 2)
+    ordering = np.zeros(n + 1, dtype=np.int32)
+    si, sj, w = np.zeros(cap, dtype=np.int32), np.zeros(cap, dtype=np.int32), np.zeros(cap, dtype=np.float64)
+    sup = np.zeros(cap, dtype=np.int32)
+    rk = np.zeros(max(1, R), dtype=np.int64)
+    ro = np.zeros((max(1, R), n + 1), dtype=np.int32) if replicate_orderings else None
+    t = np.zeros(5, dtype=np.float64)
+    kept = ctypes.c_int64()
+    ip = ctypes.POINTER(ctypes.c_int32)
+    _check(lib().fnn_bootstrap(ctypes.byref(o), codes.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)), n, L, m, u, R, int(boot_seed),
+                               float(cutoff), ordering.ctypes.data_as(ip), si.ctypes.data_as(ip), sj.ctypes.data_as(ip), _dp(w),
+                               sup.ctypes.data_as(ip), cap, ctypes.byref(kept), None if ro is None else ro.ctypes.data_as(ip),
+                               rk.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _dp(t)))
+    k = kept.value
+    times = {"distances_ms": float(t[0]), "ordering_ms": float(t[1]), "split_weights_ms": float(t[2]), "matching_ms": float(t[3]),
+             "cg_iters": int(t[4])}
+    return Bootstrap(ordering, si[:k].copy(), sj[:k].copy(), w[:k].copy(), sup[:k].copy(), rk[:R].copy(),
+                     None if ro is None else ro[:R].copy(), times)
 
 
 def csw_matvec(which, v, n, variant="default", **opts):

@@ -1493,9 +1493,8 @@ extern "C" int fnn_csw_matvec(const fnn_opts* o, int32_t which, const double* v,
     return rc;
 }
 
-// shared driver of the two B2 entry points: upload, permute to circular-position order, solve; leaves x on the device
-static int solve_split_weights(Csw& c, const fnn_opts* o, const int32_t* ordering, const double* d_upper, int64_t n,
-                               bool d_upper_on_device = false) {
+// allocation and solver configuration for n taxa, once per workspace
+static int csw_prepare(Csw& c, const fnn_opts* o, int64_t n) {
     c.n = (int)n; c.np = n * (n - 1) / 2; c.nblk = (c.np + 1023) / 1024;
     c.literal = (o && o->reserved[4] == 2) ? 1 : 0;
     if (c.literal && n > lit::MAX_N) { fnn::set_error("split weights: the literal-order validation mode covers n <= %d", lit::MAX_N); return FNN_E_ARG; }
@@ -1518,15 +1517,39 @@ static int solve_split_weights(Csw& c, const fnn_opts* o, const int32_t* orderin
             c.persistent_grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)sms * per_sm, want));
         }
     }
+    return FNN_OK;
+}
+
+// a prepared workspace back in the state csw_prepare leaves it in, for the next solve of the same size
+static int csw_reset(Csw& c) {
+    FNN_CUDA(cudaMemsetAsync(c.sc, 0, sizeof(Scalars), c.st));
+    FNN_CUDA(cudaMemsetAsync(c.sel, 0, sizeof(SelState), c.st));
+    memset(c.h_sc, 0, sizeof(Scalars));
+    c.cg_calls = c.outer = c.inner = c.launches = 0;
+    return FNN_OK;
+}
+
+// upload, permute to circular-position order, solve; leaves x on the device
+static int csw_solve(Csw& c, const fnn_opts* o, const int32_t* ordering, const double* d_upper, bool d_upper_on_device) {
+    const int64_t n = c.n;
     int* d_ord = reinterpret_cast<int*>(c.tie_rank);   // scratch: free until the first 60 % collapse
     FNN_CUDA(cudaMemcpyAsync(d_ord, ordering, sizeof(int) * (n + 1), cudaMemcpyHostToDevice, c.st));
     FNN_CUDA(cudaMemcpyAsync(c.r, d_upper, sizeof(double) * c.np, d_upper_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice,
                              c.st));   // r as staging
     k_setup_d<<<c.grid_rows(), 256, 0, c.st>>>(c.r, d_ord, c.d, c.n);
     const bool unconstrained = o && o->reserved[3] == 1;
-    if (unconstrained) k_unconstrained<<<c.grid_rows(), 256, 0, c.st>>>(c.d, c.x, c.n);
-    else rc = active_conjugate(c);
-    return rc;
+    if (unconstrained) {
+        k_unconstrained<<<c.grid_rows(), 256, 0, c.st>>>(c.d, c.x, c.n);
+        return FNN_OK;
+    }
+    return active_conjugate(c);
+}
+
+// shared driver of the B2 entry points; leaves x on the device
+static int solve_split_weights(Csw& c, const fnn_opts* o, const int32_t* ordering, const double* d_upper, int64_t n) {
+    int rc = csw_prepare(c, o, n);
+    if (rc) return rc;
+    return csw_solve(c, o, ordering, d_upper, false);
 }
 
 static int check_b2_args(const fnn_opts* o, const int32_t* ordering, const double* d_upper, int64_t n) {
@@ -1616,33 +1639,51 @@ __global__ void k_compact(const double* __restrict__ x, const int* __restrict__ 
         }
 }
 
-// FastNN.java:455-466 on the device: keep the splits whose weight exceeds `cutoff`, compacted in (i, j) order.
-static int emit_kept_splits(Csw& c, int64_t n, double cutoff, int32_t* split_i, int32_t* split_j, double* weight, int64_t max_out,
-                            int64_t* n_out) {
+// FastNN.java:455-466 on the device: flag the splits whose weight exceeds `cutoff` and count them (one host read)
+static int count_kept(Csw& c, double cutoff, long long* kept) {
     k_flag_above<<<c.grid1d(c.np, 256), 256, 0, c.st>>>(c.x, c.tie_flag, c.np, cutoff);
     k_flag_local<<<(unsigned)c.nblk, 1024, 0, c.st>>>(c.tie_flag, c.np, c.tie_rank, c.blk_sum, nullptr);
     k_flag_blockscan<<<1, 1024, 0, c.st>>>(c.blk_sum, c.nblk, c.sel, nullptr);
     FNN_CUDA(cudaMemcpyAsync(c.h_sel, c.sel, sizeof(SelState), cudaMemcpyDeviceToHost, c.st));
     FNN_CUDA(cudaStreamSynchronize(c.st));
-    const long long kept = c.h_sel->flag_total;
-    *n_out = kept;
-    if (kept > max_out) { fnn::set_error("weighted splits: %lld splits kept, room for %lld", kept, (long long)max_out); return FNN_E_ARG; }
-    if (kept > 0) {
-        // the solver's scratch vectors are free now: p holds the kept weights, the first kept ints of w their packed indices
-        int* d_idx = reinterpret_cast<int*>(c.w);
-        k_compact<<<c.grid1d(c.np, 256), 256, 0, c.st>>>(c.x, c.tie_flag, c.tie_rank, c.blk_sum, c.np, d_idx, c.p);
-        std::vector<int> idx_h((size_t)kept);
-        FNN_CUDA(cudaMemcpyAsync(idx_h.data(), d_idx, sizeof(int) * (size_t)kept, cudaMemcpyDeviceToHost, c.st));
-        FNN_CUDA(cudaMemcpyAsync(weight, c.p, sizeof(double) * (size_t)kept, cudaMemcpyDeviceToHost, c.st));
-        FNN_CUDA(cudaStreamSynchronize(c.st));
-        int64_t i = 0;
-        for (long long k = 0; k < kept; ++k) {   // packed index -> (i, j); indices are increasing, so i only moves forward
-            while (row_start(n, i + 1) <= idx_h[k]) ++i;
-            split_i[k] = (int32_t)i;
-            split_j[k] = (int32_t)(idx_h[k] - row_start(n, i) + i + 1);
-        }
+    *kept = c.h_sel->flag_total;
+    return FNN_OK;
+}
+
+// the solver's scratch vectors are free now: the first kept ints of w get the flagged packed indices in (i, j) order,
+// p their weights
+static int* compact_kept(Csw& c) {
+    int* d_idx = reinterpret_cast<int*>(c.w);
+    k_compact<<<c.grid1d(c.np, 256), 256, 0, c.st>>>(c.x, c.tie_flag, c.tie_rank, c.blk_sum, c.np, d_idx, c.p);
+    return d_idx;
+}
+
+// the compacted splits to the host as (i, j, weight)
+static int copy_kept(Csw& c, int64_t n, long long kept, int32_t* split_i, int32_t* split_j, double* weight) {
+    if (kept <= 0) return FNN_OK;
+    std::vector<int> idx_h((size_t)kept);
+    FNN_CUDA(cudaMemcpyAsync(idx_h.data(), c.w, sizeof(int) * (size_t)kept, cudaMemcpyDeviceToHost, c.st));
+    FNN_CUDA(cudaMemcpyAsync(weight, c.p, sizeof(double) * (size_t)kept, cudaMemcpyDeviceToHost, c.st));
+    FNN_CUDA(cudaStreamSynchronize(c.st));
+    int64_t i = 0;
+    for (long long k = 0; k < kept; ++k) {   // packed index -> (i, j); indices are increasing, so i only moves forward
+        while (row_start(n, i + 1) <= idx_h[k]) ++i;
+        split_i[k] = (int32_t)i;
+        split_j[k] = (int32_t)(idx_h[k] - row_start(n, i) + i + 1);
     }
     return FNN_OK;
+}
+
+// keep x > cutoff, compacted in (i, j) order, and copy them out
+static int emit_kept_splits(Csw& c, int64_t n, double cutoff, int32_t* split_i, int32_t* split_j, double* weight, int64_t max_out,
+                            int64_t* n_out) {
+    long long kept = 0;
+    int rc = count_kept(c, cutoff, &kept);
+    if (rc) return rc;
+    *n_out = kept;
+    if (kept > max_out) { fnn::set_error("weighted splits: %lld splits kept, room for %lld", kept, (long long)max_out); return FNN_E_ARG; }
+    if (kept > 0) compact_kept(c);
+    return copy_kept(c, n, kept, split_i, split_j, weight);
 }
 
 extern "C" int fnn_weighted_splits(const fnn_opts* o, const int32_t* ordering, const double* d_upper, int64_t n, double cutoff,
@@ -1669,9 +1710,90 @@ __global__ void k_pack_upper(const double* __restrict__ D, int64_t ld, int n, do
     for (int j = i + 1 + blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) out[rs + (j - i - 1)] = D[(int64_t)i * ld + j];
 }
 
-// The whole network in one call (SURVEY §8b "optional fnn_network"): FastNN.main's ordering stage and split stage chained
-// with the distances kept on the device - the packed upper triangle is taken from the device matrix before the ordering
-// consumes it, so the split stage uploads nothing but the ordering.
+// FastNN.main's ordering stage and split stage chained with the distances kept on the device (fnn_network, fnn_bootstrap):
+// the packed upper triangle is taken from the device matrix before the ordering consumes it, so the split stage uploads
+// nothing but the ordering.  The workspace serves every run of the same n.
+struct NetChain {
+    fnn_opts o;
+    int64_t n = 0;
+    Csw c;
+    double* d_upper = nullptr;
+    bool used = false;
+};
+
+int fnn_chain_create_(const fnn_opts* o, int64_t n, NetChain** out) {
+    NetChain* w = new NetChain();
+    if (o) w->o = *o;
+    else fnn_default_opts(&w->o);
+    w->n = n;
+    int rc = csw_prepare(w->c, &w->o, n);
+    if (!rc && cudaMalloc((void**)&w->d_upper, sizeof(double) * (size_t)w->c.np) != cudaSuccess) {
+        fnn::set_error("split weights: cudaMalloc of the packed triangle failed: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = FNN_E_CUDA;
+    }
+    if (rc) { fnn_chain_destroy_(w); return rc; }
+    *out = w;
+    return FNN_OK;
+}
+
+void fnn_chain_destroy_(NetChain* w) {
+    if (!w) return;
+    w->c.release();
+    if (w->d_upper) cudaFree(w->d_upper);
+    delete w;
+}
+
+int fnn_chain_run_(NetChain* w, fnn_ctx* ctx, double cutoff, int32_t* ordering_out, int64_t* kept, ChainTimes* tm) {
+    const int64_t n = w->n;
+    Csw& c = w->c;
+    double* dD; int64_t ld;
+    fnn_ctx_matrix_ptr(ctx, &dD, &ld);
+    cudaStream_t cs = fnn_ctx_stream_(ctx);
+    DevEvent p0, p1, s0, s1;
+    if (tm) {
+        FNN_CUDA(p0.create()); FNN_CUDA(p1.create()); FNN_CUDA(s0.create()); FNN_CUDA(s1.create());
+        FNN_CUDA(cudaEventRecord(p0, cs));
+    }
+    k_pack_upper<<<dim3((unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, 64)), (unsigned)(n - 1)), 256, 0, cs>>>(dD, ld, (int)n, w->d_upper);
+    FNN_CUDA(cudaGetLastError());
+    if (tm) FNN_CUDA(cudaEventRecord(p1, cs));
+    FNN_CUDA(cudaStreamSynchronize(cs));
+    int rc = fnn_ctx_order(ctx, ordering_out);
+    if (rc) return rc;
+    if (w->used) { rc = csw_reset(c); if (rc) return rc; }
+    w->used = true;
+    if (tm) FNN_CUDA(cudaEventRecord(s0, c.st));
+    rc = csw_solve(c, &w->o, ordering_out, w->d_upper, true);
+    if (rc) return rc;
+    long long k = 0;
+    rc = count_kept(c, cutoff, &k);
+    if (rc) return rc;
+    *kept = k;
+    if (k > 0) compact_kept(c);
+    FNN_CUDA(cudaGetLastError());
+    if (tm) {
+        FNN_CUDA(cudaEventRecord(s1, c.st));
+        FNN_CUDA(cudaMemcpyAsync(c.h_sc, c.sc, sizeof(Scalars), cudaMemcpyDeviceToHost, c.st));
+        FNN_CUDA(cudaStreamSynchronize(c.st));
+        fnn_stats st;
+        fnn_ctx_stats(ctx, &st);
+        float a = 0, b = 0;
+        cudaEventElapsedTime(&a, p0, p1);
+        cudaEventElapsedTime(&b, s0, s1);
+        tm->order_ms = st.order_ms;
+        tm->csw_ms = (double)a + (double)b;
+        tm->cg_iters = c.h_sc->iters_total;
+    }
+    return FNN_OK;
+}
+
+const int* fnn_chain_kept_idx_(NetChain* w) { return reinterpret_cast<const int*>(w->c.w); }
+cudaStream_t fnn_chain_stream_(NetChain* w) { return w->c.st; }
+int fnn_chain_copy_kept_(NetChain* w, int64_t kept, int32_t* split_i, int32_t* split_j, double* weight) {
+    return copy_kept(w->c, w->n, kept, split_i, split_j, weight);
+}
+
+// The whole network in one call (SURVEY §8b "optional fnn_network").
 extern "C" int fnn_network(const fnn_opts* o, const double* D_rowmajor, int64_t n, double cutoff, int32_t* ordering_out,
                            int32_t* split_i, int32_t* split_j, double* weight, int64_t max_out, int64_t* n_out) {
     if (!D_rowmajor || !ordering_out || !split_i || !split_j || !weight || !n_out || n < 4 || n > 20000) {
@@ -1681,30 +1803,21 @@ extern "C" int fnn_network(const fnn_opts* o, const double* D_rowmajor, int64_t 
     fnn_ctx* ctx = nullptr;
     int rc = fnn_ctx_create(o, n, &ctx);
     if (rc) return rc;
-    double* d_upper = nullptr;
-    rc = [&]() -> int {
-        int r = fnn_ctx_load_host(ctx, D_rowmajor);
-        if (r) return r;
-        double* dD; int64_t ld;
-        fnn_ctx_matrix_ptr(ctx, &dD, &ld);
-        const int64_t np = n * (n - 1) / 2;
-        FNN_CUDA(cudaMalloc((void**)&d_upper, sizeof(double) * np));
-        cudaStream_t cs = fnn_ctx_stream_(ctx);
-        k_pack_upper<<<dim3((unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, 64)), (unsigned)(n - 1)), 256, 0, cs>>>(dD, ld, (int)n, d_upper);
-        FNN_CUDA(cudaGetLastError());
-        FNN_CUDA(cudaStreamSynchronize(cs));
-        r = fnn_ctx_order(ctx, ordering_out);
-        return r;
-    }();
-    fnn_ctx_destroy(ctx);
+    NetChain* w = nullptr;
+    rc = fnn_ctx_load_host(ctx, D_rowmajor);
+    if (!rc) rc = fnn_chain_create_(o, n, &w);
+    int64_t kept = 0;
+    if (!rc) rc = fnn_chain_run_(w, ctx, cutoff, ordering_out, &kept, nullptr);
     if (!rc) {
-        Csw c;
-        rc = solve_split_weights(c, o, ordering_out, d_upper, n, true);
-        if (!rc) {
-            rc = emit_kept_splits(c, n, cutoff, split_i, split_j, weight, max_out, n_out);
+        *n_out = kept;
+        if (kept > max_out) {
+            fnn::set_error("weighted splits: %lld splits kept, room for %lld", (long long)kept, (long long)max_out);
+            rc = FNN_E_ARG;
+        } else {
+            rc = fnn_chain_copy_kept_(w, kept, split_i, split_j, weight);
         }
-        c.release();
     }
-    if (d_upper) cudaFree(d_upper);
+    fnn_chain_destroy_(w);
+    fnn_ctx_destroy(ctx);
     return rc;
 }

@@ -1,6 +1,7 @@
 // fnn_dist.cu — pairwise distances of a nucleotide alignment on the device (P, JC69, K2P; pairwise deletion), written
-// straight into a device matrix: the context's own (fnn_ctx_load_alignment) or a scratch buffer copied back to the host
-// (fnn_distances).  DESIGN.md §4.4.
+// straight into a device matrix: the context's own (fnn_ctx_load_alignment, fnn_bootstrap) or a scratch buffer copied back to
+// the host (fnn_distances).  DESIGN.md §4.4.  DistJob (fnn_common.h) uploads the codes once; a bootstrap replicate then
+// packs its planes through its list of drawn columns.
 //
 //   k_pack   codes (uint8, n x L, 0..4) -> three bit-planes per 64-site word and taxon.  With A=00 G=01 C=10 T=11 (hi, lo):
 //            hi = pyrimidine, lo = G or T, ok = the site holds a state.  ok is 0 past L and for padding
@@ -34,15 +35,17 @@ static_assert(16 * MT == TM, "micro-tile layout");
 
 const char* model_name(int32_t model) { return model == FNN_DIST_P ? "p" : (model == FNN_DIST_JC69 ? "jc69" : "k2p"); }
 
-// one warp per (taxon, word): each lane maps two sites, three ballots give the word's planes
-__global__ void k_pack(const uint8_t* __restrict__ codes, int64_t n, int64_t L, int64_t W, int64_t np,
+// one warp per (taxon, word): each lane maps two sites, three ballots give the word's planes.  sites (optional, L entries):
+// site s of the packed alignment is column sites[s] of codes (a bootstrap replicate); NULL = column s.
+__global__ void k_pack(const uint8_t* __restrict__ codes, int64_t n, int64_t L, int64_t W, int64_t np, const int32_t* __restrict__ sites,
                        unsigned long long* __restrict__ planes, int* __restrict__ bad) {
     const int lane = threadIdx.x & 31;
     const int64_t warps = (int64_t)gridDim.x * (blockDim.x / 32);
     for (int64_t u = (int64_t)blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32; u < n * W; u += warps) {
         const int64_t t = u / W, w = u - t * W;
         const int64_t s0 = w * 64 + lane, s1 = s0 + 32;
-        const unsigned c0 = s0 < L ? codes[t * L + s0] : 4u, c1 = s1 < L ? codes[t * L + s1] : 4u;
+        const unsigned c0 = s0 < L ? codes[t * L + (sites ? sites[s0] : s0)] : 4u;
+        const unsigned c1 = s1 < L ? codes[t * L + (sites ? sites[s1] : s1)] : 4u;
         if (c0 > 4u || c1 > 4u) atomicOr(bad, 1);
         const bool ok0 = c0 < 4u, ok1 = c1 < 4u;
         const unsigned hi0 = __ballot_sync(0xffffffffu, ok0 && (c0 & 1u)), hi1 = __ballot_sync(0xffffffffu, ok1 && (c1 & 1u));
@@ -185,11 +188,9 @@ __global__ void __launch_bounds__(THREADS) k_pairs(const unsigned long long* __r
     }
 }
 
-struct DistTimes {
-    float upload_ms = 0, pack_ms = 0, pairs_ms = 0;
-};
+}  // namespace
 
-int check_args(const char* who, const uint8_t* codes, int64_t n, int64_t sites, int32_t model, double undef) {
+int fnn_dist_check_args_(const char* who, const uint8_t* codes, int64_t n, int64_t sites, int32_t model, double undef) {
     if (!codes || n < 1 || n > 2000000 || sites < 1 || sites > INT32_MAX) {
         fnn::set_error("%s: need codes, 1 <= n <= 2000000 and 1 <= sites <= 2^31-1 (got n = %lld, sites = %lld)", who, (long long)n,
                        (long long)sites);
@@ -203,41 +204,56 @@ int check_args(const char* who, const uint8_t* codes, int64_t n, int64_t sites, 
     return FNN_OK;
 }
 
-// v, m, s of one pair on the host, for the error message
-void host_counts(const uint8_t* codes, int64_t sites, int64_t i, int64_t j, long long* v, long long* m, long long* s) {
+namespace {
+
+// v, m, s of one pair on the host, for the error message (sites: the replicate's columns, NULL = all)
+void host_counts(const uint8_t* codes, int64_t L, const int32_t* sites, int64_t i, int64_t j, long long* v, long long* m, long long* s) {
     *v = *m = *s = 0;
-    const uint8_t *x = codes + i * sites, *y = codes + j * sites;
-    for (int64_t k = 0; k < sites; ++k) {
-        if (x[k] < 4 && y[k] < 4) {
+    const uint8_t *x = codes + i * L, *y = codes + j * L;
+    for (int64_t k = 0; k < L; ++k) {
+        const int64_t col = sites ? sites[k] : k;
+        if (x[col] < 4 && y[col] < 4) {
             ++*v;
-            if (x[k] != y[k]) { ++*m; if ((x[k] ^ y[k]) == 2) ++*s; }
+            if (x[col] != y[col]) { ++*m; if ((x[col] ^ y[col]) == 2) ++*s; }
         }
     }
 }
 
-// The whole device computation into dD (leading dimension ld) on `stream`.
-int dist_run(const char* who, cudaStream_t stream, int sms, const uint8_t* codes, int64_t n, int64_t L, int32_t model, double undef,
-             double* dD, int64_t ld, DistTimes* tm) {
-    const int64_t W = (L + 63) / 64, stages = (W + BK - 1) / BK, np = (n + TM - 1) / TM * TM, nt = np / TM;
+}  // namespace
+
+int DistJob::upload(cudaStream_t stream_, int sms_, const uint8_t* codes_, int64_t n_, int64_t L_, bool resample, DistTimes* tm) {
+    stream = stream_; sms = sms_; codes = codes_; n = n_; L = L_;
+    const int64_t W = (L + 63) / 64, stages = (W + BK - 1) / BK, np = (n + TM - 1) / TM * TM;
     const size_t plane_bytes = sizeof(unsigned long long) * PLANES * (size_t)(stages * BK) * (size_t)np;
-    uint8_t* d_codes = nullptr;
-    unsigned long long* d_planes = nullptr;
-    unsigned long long* d_flags = nullptr;   // [0] = first undefined pair key, [1] = bad-code flag
-    DevScratch scratch;
     FNN_CUDA(scratch.alloc((void**)&d_codes, (size_t)n * (size_t)L));
     FNN_CUDA(scratch.alloc((void**)&d_planes, plane_bytes));
     FNN_CUDA(scratch.alloc((void**)&d_flags, 2 * sizeof(unsigned long long)));
-    const unsigned long long init[2] = {~0ull, 0ull};
-    FNN_CUDA(cudaMemcpyAsync(d_flags, init, sizeof(init), cudaMemcpyHostToDevice, stream));
-    FNN_CUDA(cudaMemsetAsync(d_planes, 0, plane_bytes, stream));   // tail words and padding taxa: ok = 0
-    DevEvent e0, e1, e2, e3;
-    FNN_CUDA(e0.create()); FNN_CUDA(e1.create()); FNN_CUDA(e2.create()); FNN_CUDA(e3.create());
+    if (resample) FNN_CUDA(scratch.alloc((void**)&d_sites, sizeof(int32_t) * (size_t)L));
+    // tail words and padding taxa: ok = 0.  k_pack never writes them, so this holds for every later pack.
+    FNN_CUDA(cudaMemsetAsync(d_planes, 0, plane_bytes, stream));
+    DevEvent e0, e1;
+    FNN_CUDA(e0.create()); FNN_CUDA(e1.create());
     FNN_CUDA(cudaEventRecord(e0, stream));
     FNN_CUDA(cudaMemcpyAsync(d_codes, codes, (size_t)n * (size_t)L, cudaMemcpyHostToDevice, stream));
     FNN_CUDA(cudaEventRecord(e1, stream));
+    FNN_CUDA(cudaStreamSynchronize(stream));
+    if (tm) cudaEventElapsedTime(&tm->upload_ms, e0, e1);
+    return FNN_OK;
+}
+
+int DistJob::run(const char* who, const char* where, int32_t model, double undef, const int32_t* sites, double* dD, int64_t ld,
+                 DistTimes* tm) {
+    const int64_t W = (L + 63) / 64, stages = (W + BK - 1) / BK, np = (n + TM - 1) / TM * TM, nt = np / TM;
+    if (sites && !d_sites) { fnn::set_error("%s: no site list buffer", who); return FNN_E_STATE; }
+    const unsigned long long init[2] = {~0ull, 0ull};   // [0] = first undefined pair key, [1] = bad-code flag
+    FNN_CUDA(cudaMemcpyAsync(d_flags, init, sizeof(init), cudaMemcpyHostToDevice, stream));
+    if (sites) FNN_CUDA(cudaMemcpyAsync(d_sites, sites, sizeof(int32_t) * (size_t)L, cudaMemcpyHostToDevice, stream));
+    DevEvent e1, e2, e3;
+    FNN_CUDA(e1.create()); FNN_CUDA(e2.create()); FNN_CUDA(e3.create());
+    FNN_CUDA(cudaEventRecord(e1, stream));
     const int64_t units = n * W;
     const int pack_grid = (int)std::min<int64_t>((units + 7) / 8, (int64_t)sms * 64);
-    k_pack<<<pack_grid, 256, 0, stream>>>(d_codes, n, L, W, np, d_planes, (int*)(d_flags + 1));
+    k_pack<<<pack_grid, 256, 0, stream>>>(d_codes, n, L, W, np, sites ? d_sites : nullptr, d_planes, (int*)(d_flags + 1));
     FNN_CUDA(cudaGetLastError());
     FNN_CUDA(cudaEventRecord(e2, stream));
     const int64_t tiles = nt * (nt + 1) / 2;
@@ -252,7 +268,6 @@ int dist_run(const char* who, cudaStream_t stream, int sms, const uint8_t* codes
     FNN_CUDA(cudaMemcpyAsync(flags, d_flags, sizeof(flags), cudaMemcpyDeviceToHost, stream));
     FNN_CUDA(cudaStreamSynchronize(stream));
     if (tm) {
-        cudaEventElapsedTime(&tm->upload_ms, e0, e1);
         cudaEventElapsedTime(&tm->pack_ms, e1, e2);
         cudaEventElapsedTime(&tm->pairs_ms, e2, e3);
     }
@@ -260,21 +275,19 @@ int dist_run(const char* who, cudaStream_t stream, int sms, const uint8_t* codes
     if (flags[0] != ~0ull) {
         const int64_t i = (int64_t)(flags[0] / (unsigned long long)n), j = (int64_t)(flags[0] % (unsigned long long)n);
         long long v, m, s;
-        host_counts(codes, L, i, j, &v, &m, &s);
-        fnn::set_error("%s: the %s distance of pair (%lld, %lld) is undefined: v = %lld comparable sites, m = %lld differences, "
-                       "s = %lld transitions; pass a finite undefined_value >= 0 to substitute it", who, model_name(model),
+        host_counts(codes, L, sites, i, j, &v, &m, &s);
+        fnn::set_error("%s: %sthe %s distance of pair (%lld, %lld) is undefined: v = %lld comparable sites, m = %lld differences, "
+                       "s = %lld transitions; pass a finite undefined_value >= 0 to substitute it", who, where, model_name(model),
                        (long long)i, (long long)j, v, m, s);
         return FNN_E_ARG;
     }
     return FNN_OK;
 }
 
-}  // namespace
-
 extern "C" int fnn_ctx_load_alignment(fnn_ctx* c, const uint8_t* codes, int64_t sites, int32_t model, double undefined_value) {
     if (!c) { fnn::set_error("fnn_ctx_load_alignment: null context"); return FNN_E_ARG; }
     const int64_t n = fnn_ctx_n_(c);
-    int rc = check_args("fnn_ctx_load_alignment", codes, n, sites, model, undefined_value);
+    int rc = fnn_dist_check_args_("fnn_ctx_load_alignment", codes, n, sites, model, undefined_value);
     if (rc) return rc;
     FNN_CUDA(cudaSetDevice(fnn_ctx_device_(c)));
     double* dD;
@@ -282,7 +295,9 @@ extern "C" int fnn_ctx_load_alignment(fnn_ctx* c, const uint8_t* codes, int64_t 
     fnn_ctx_matrix_ptr(c, &dD, &ld);
     fnn_ctx_mark_unloaded_(c);   // the matrix is overwritten; it counts as loaded only once the call succeeds
     DistTimes tm;
-    rc = dist_run("fnn_ctx_load_alignment", fnn_ctx_stream_(c), fnn_ctx_sms_(c), codes, n, sites, model, undefined_value, dD, ld, &tm);
+    DistJob job;
+    rc = job.upload(fnn_ctx_stream_(c), fnn_ctx_sms_(c), codes, n, sites, false, &tm);
+    if (!rc) rc = job.run("fnn_ctx_load_alignment", "", model, undefined_value, nullptr, dD, ld, &tm);
     if (rc) return rc;
     fnn_stats* st = fnn_ctx_stats_(c);
     st->h2d_ms = tm.upload_ms;
@@ -294,7 +309,7 @@ extern "C" int fnn_ctx_load_alignment(fnn_ctx* c, const uint8_t* codes, int64_t 
 
 extern "C" int fnn_distances(const fnn_opts* o, const uint8_t* codes, int64_t n, int64_t sites, int32_t model, double undefined_value,
                              double* D_out) {
-    int rc = check_args("fnn_distances", codes, n, sites, model, undefined_value);
+    int rc = fnn_dist_check_args_("fnn_distances", codes, n, sites, model, undefined_value);
     if (rc) return rc;
     if (!D_out) { fnn::set_error("fnn_distances: null D_out"); return FNN_E_ARG; }
     int cnt = 0;
@@ -314,7 +329,9 @@ extern "C" int fnn_distances(const fnn_opts* o, const uint8_t* codes, int64_t n,
     double* dD = nullptr;
     DevScratch scratch;
     FNN_CUDA(scratch.alloc((void**)&dD, sizeof(double) * (size_t)n * (size_t)n));
-    rc = dist_run("fnn_distances", stream, sms, codes, n, sites, model, undefined_value, dD, n, nullptr);
+    DistJob job;
+    rc = job.upload(stream, sms, codes, n, sites, false, nullptr);
+    if (!rc) rc = job.run("fnn_distances", "", model, undefined_value, nullptr, dD, n, nullptr);
     if (rc) return rc;
     FNN_CUDA(cudaMemcpyAsync(D_out, dD, sizeof(double) * (size_t)n * (size_t)n, cudaMemcpyDeviceToHost, stream));
     FNN_CUDA(cudaStreamSynchronize(stream));

@@ -101,9 +101,23 @@ extern "C" int fnn_java_double_to_string(double v, char* out, int64_t out_len) {
 extern "C" int fnn_write_nexus(const char* path, int64_t n, const char* names, int64_t name_stride, const double* D,
                                const int32_t* ordering, const int32_t* split_i, const int32_t* split_j, const double* weight,
                                int64_t n_splits, int threads) {
+    return fnn_write_nexus_support(path, n, names, name_stride, D, ordering, split_i, split_j, weight, nullptr, 0, n_splits, threads);
+}
+
+extern "C" int fnn_write_nexus_support(const char* path, int64_t n, const char* names, int64_t name_stride, const double* D,
+                                       const int32_t* ordering, const int32_t* split_i, const int32_t* split_j, const double* weight,
+                                       const int32_t* support, int32_t replicates, int64_t n_splits, int threads) {
     if (n < 1 || !ordering || n_splits < 0 || (n_splits > 0 && (!split_i || !split_j || !weight)) || (names && name_stride < 1)) {
         fnn::set_error("fnn_write_nexus: bad arguments");
         return FNN_E_ARG;
+    }
+    if (support) {
+        if (replicates < 1) { fnn::set_error("fnn_write_nexus_support: replicates %d, need >= 1", replicates); return FNN_E_ARG; }
+        for (int64_t k = 0; k < n_splits; ++k)
+            if (support[k] < 0 || support[k] > replicates) {
+                fnn::set_error("fnn_write_nexus_support: support[%lld] = %d is outside 0..%d", (long long)k, support[k], replicates);
+                return FNN_E_ARG;
+            }
     }
     for (int64_t k = 0; k < n_splits; ++k)
         if (split_i[k] < 0 || split_j[k] <= split_i[k] || split_j[k] >= n) {
@@ -191,7 +205,8 @@ extern "C" int fnn_write_nexus(const char* path, int64_t n, const char* names, i
     put_int(s, n);
     s += " nsplits=";
     put_int(s, n_splits);
-    s += ";\nFORMAT labels=no weights=yes confidences=no intervals=no;\nPROPERTIES fit=-1.0 cyclic;\nCYCLE";
+    s += support ? ";\nFORMAT labels=no weights=yes confidences=yes intervals=no;\nPROPERTIES fit=-1.0 cyclic;\nCYCLE"
+                 : ";\nFORMAT labels=no weights=yes confidences=no intervals=no;\nPROPERTIES fit=-1.0 cyclic;\nCYCLE";
     for (int64_t i = 1; i <= n; ++i) { s += ' '; put_int(s, ordering[i]); }
     s += ";\nMATRIX\n";
     std::vector<uint64_t> bits((size_t)(n + 64) / 64 + 1);
@@ -207,6 +222,10 @@ extern "C" int fnn_write_nexus(const char* path, int64_t n, const char* names, i
         s += "] \t ";
         s.append(b, (size_t)java_double(weight[k], b));
         s += " \t ";
+        if (support) {   // the confidence column: percent of the replicates that contain the split
+            s.append(b, (size_t)java_double((100.0 * (double)support[k]) / (double)replicates, b));
+            s += " \t ";
+        }
         // members in increasing taxon id (BitSet.nextSetBit order, :76-80)
         int lo = INT32_MAX, hi = 0;
         for (int64_t q = i + 1; q <= j; ++q) {

@@ -198,6 +198,13 @@ int fnn_write_nexus(const char* path, int64_t n, const char* names, int64_t name
                     const int32_t* ordering, const int32_t* split_i, const int32_t* split_j, const double* weight,
                     int64_t n_splits, int threads);
 int fnn_java_double_to_string(double v, char* out, int64_t out_len);
+/* fnn_write_nexus with bootstrap support (fnn_bootstrap): support[k] (0..replicates) for split k.  The FORMAT line then says
+ * confidences=yes and every split line carries the confidence c = (100.0 * support[k]) / replicates, formatted like the
+ * weight, between the weight and the members: `[k, size=s] \t w \t c \t members,`.  support NULL = fnn_write_nexus, byte for
+ * byte (replicates is then ignored). */
+int fnn_write_nexus_support(const char* path, int64_t n, const char* names, int64_t name_stride, const double* D_rowmajor,
+                            const int32_t* ordering, const int32_t* split_i, const int32_t* split_j, const double* weight,
+                            const int32_t* support, int32_t replicates, int64_t n_splits, int threads);
 
 /* B1 + B2 chained with the distances kept on the device (FastNN.main without -order, FastNN.java:378-466): ordering, then
  * split weights of the SAME matrix (its packed upper triangle is taken on the device before the ordering consumes it),
@@ -263,6 +270,30 @@ int fnn_ctx_load_alignment(fnn_ctx* c, const uint8_t* codes, int64_t sites, int3
 /* Host in, host out: D_out (n*n, row-major) on device opts->device (o NULL = defaults); needs no context. */
 int fnn_distances(const fnn_opts* o, const uint8_t* codes, int64_t n, int64_t sites, int32_t model, double undefined_value,
                   double* D_out);
+
+/* ---- bootstrap support of the splits of an alignment's network (DESIGN.md §4.5) -------------------------------------
+ * Input: codes (n x sites) and model / undefined_value as for fnn_distances; the ordering options of o (mode, mult, seed,
+ * canonical_fallback; o NULL = defaults); 4 <= n <= 20000 as for fnn_network; replicates = R >= 1.
+ *   Original network: the distances of the alignment as given, then ordering, split weights and the kept splits (x > cutoff),
+ *     bit-identical to fnn_network on fnn_distances(codes): ordering_out (n+1), split_i / split_j / weight (*n_out of them,
+ *     FNN_E_ARG beyond max_out).
+ *   Resampling: one java.util.Random(boot_seed) stream; replicate r takes the r-th run of `sites` values of nextInt(sites)
+ *     (the LCG and rejection rule of the Random modes) as its columns.  Distances depend only on counts over the columns, so
+ *     the order of the draws does not matter (they are sorted).
+ *   Replicate: distances of the resampled alignment, then an ordering with the same options (the ordering's own RNG restarts
+ *     from o->seed in every replicate, as in a fresh context), split weights and kept splits.  undefined_value applies to
+ *     every replicate; with NaN an undefined pair fails the call with FNN_E_ARG, the message naming the replicate, the pair
+ *     and its v, m, s in that replicate.
+ *   Support: support[k] (int32, 0..R) = number of replicates whose kept splits contain original split k as a bipartition of
+ *     the taxa.  Matched exactly on the device, without hashing: a replicate split's side U without taxon O[n] (O = original
+ *     ordering) is original split (i, j) iff the positions of U in O are the contiguous range i+1..j.
+ * Optional outputs (NULL = not wanted): replicate_orderings (R * (n+1)), replicate_kept (R: kept splits per replicate),
+ * times_out (5: distances, ordering, split weights and matching ms, CUDA events summed over the replicates, then the total
+ * CG iterations of the replicates' solves). */
+int fnn_bootstrap(const fnn_opts* o, const uint8_t* codes, int64_t n, int64_t sites, int32_t model, double undefined_value,
+                  int32_t replicates, int64_t boot_seed, double cutoff, int32_t* ordering_out, int32_t* split_i, int32_t* split_j,
+                  double* weight, int32_t* support, int64_t max_out, int64_t* n_out, int32_t* replicate_orderings,
+                  int64_t* replicate_kept, double* times_out);
 
 /* left-to-right fp64 sums of nrows (<=4) rows of length len, bit-identical to `for (i) s += x[i]`
  * (the accumulation order of ComputeRx / updateClusterDistances, NetMakerOriginal.java:549-561, :530-535),
